@@ -1,8 +1,9 @@
 // ahsoka_main.cpp — `Ahsoka phase` / `Ahsoka only-bubbles` with the phasing step behind the
-// C ABI.  Same options, same files, same stdout banners as reference src/polyassembly.cpp:22-176;
-// the reference's own translation units (graph.cpp, alignmentreader.cpp, argumentparser.cpp,
-// chainstoreadset.cpp) are linked unchanged, as BASELINE.json's north_star prescribes, and
-// AHSOKA_HOST=reference runs every host stage through them.  By default the stages either side of the
+// C ABI.  Same options, same files, same stdout banners as reference src/polyassembly.cpp:22-176.
+// Built with AHSOKA_REFERENCE, the reference's own translation units (graph.cpp, alignmentreader.cpp,
+// argumentparser.cpp, chainstoreadset.cpp) are linked unchanged, as BASELINE.json's north_star prescribes,
+// and AHSOKA_HOST=reference runs every host stage through them; built without them, the declarations
+// and the parser under standalone/ take their place and AHSOKA_HOST=reference exits with 69.  By default the stages either side of the
 // phasing call that cannot ingest a BASELINE-sized input (SURVEY §8 f1, f4: GFA parsing and bubble
 // detection copying node sequences at every step, the GAF reader's O(L²) strings per line, the O(B²)
 // allele-path enumeration) run through this repo's result-identical replacements (graph_native.cpp,

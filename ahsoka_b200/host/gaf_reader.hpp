@@ -17,7 +17,7 @@
 #include <unordered_map>
 #include <vector>
 
-#include "graph.hpp"   // reference header (Graph::nodes → chain ids), found through -I<reference>/src
+#include "graph.hpp"   // Graph::nodes → chain ids: the reference's header (-I<reference>/src) or standalone/graph.hpp
 
 namespace ahs_host {
 

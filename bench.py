@@ -199,6 +199,24 @@ def run_reference_arm(args):
     return 0
 
 
+DUMP_MAX_ELEMS = 1 << 19          # per array: 15 arrays x 4 MB of float64 stay under 64 MB
+
+
+def dump_outputs(res, out_dir):
+    """Every array of the result as <out_dir>/<name>.npy in float64 (the integer values are exact there), plus the three
+    counts.  An array above DUMP_MAX_ELEMS elements is replaced by the elements at a fixed, seeded, sorted sample of
+    indices, so that two builds run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: getattr(res, k) for k in res.ARRAYS}
+    arrays.update({k: np.array([getattr(res, k)]) for k in ("n_cells", "n_pairs", "n_chains_ok")})
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a).reshape(-1)
+        if a.size > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(20261020).choice(a.size, DUMP_MAX_ELEMS, replace=False))
+            a = a[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
 def _emit(line):
     """The ONE JSON line goes to the real stdout; everything else a library prints there (NCCL's version banner,
     torchrun notices) was redirected to stderr at start-up."""
@@ -215,14 +233,19 @@ def main():
     os.dup2(2, 1)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed passes of every single-device leg (the N > 1 multi-device check times 3 calls)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="cfg2")
     ap.add_argument("--scale", type=float, default=1.0)
     ap.add_argument("--ref-chains", type=int, default=0, help="chains in the reference-arm sample (0 = sized from steps + warmup)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result arrays of the last timed pass as DIR/<name>.npy (float64; rank 0's batch when N > 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the result of the b200 path")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":
@@ -348,7 +371,7 @@ def main():
     api.unpin_batch(batch)
     api.phase_batch(batch, device=local, copy=False).release()
     pg_times = []
-    for _ in range(max(2, min(args.steps, 5))):
+    for _ in range(args.steps):
         t0 = time.perf_counter(); r2 = api.phase_batch(batch, device=local, copy=False); pg_times.append(time.perf_counter() - t0)
         r2.release()
     e2e_pageable_ms = 1e3 * sum(pg_times) / len(pg_times)
@@ -423,6 +446,8 @@ def main():
         line["per_rank"] = per_rank
     if not args.no_cpu_baseline and world == 1:          # reported on rank 0 at N=1 only
         line["cpu_baseline"] = cpu_port_baseline(batch)
+    if args.dump_outputs:
+        dump_outputs(res, args.dump_outputs)
     _emit(line)
     if dist is not None:
         dist.destroy_process_group()

@@ -8,9 +8,10 @@ Ahsoka-owned stage (projection, filter, ordering, coverage, consensus, re-packin
 the text format of README.md:28-42) to the reference text itself.
 
   * not gpu: host drop-in (flatten + emission) with the CPU oracle behind the C ABI
-             (oracle/_ref/Ahsoka_flat_oracle) must reproduce those files byte for byte;
+             (oracle/_ref/Ahsoka_flat_oracle, or oracle/_ref/Ahsoka_flat_oracle_standalone when the
+             original's sources were not given at build time) must reproduce those files byte for byte;
   * gpu:     the same drop-in with the CUDA library behind the C ABI (ahsoka_b200/bin/Ahsoka_b200).
-Neither test reads /root/reference at run time (the binaries are prebuilt and travel to the GPU box).
+Neither test reads the original sources at run time (the binaries are built from them once, with AHSOKA_REFERENCE set).
 """
 import json
 import os
@@ -22,6 +23,9 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 REF_DIR = os.path.join(ROOT, "oracle", "_ref")
+# the drop-in with the CPU oracle behind the C ABI: linked with the original's host stages if built with AHSOKA_REFERENCE
+FLAT_ORACLE = next((p for p in (os.path.join(REF_DIR, "Ahsoka_flat_oracle"), os.path.join(REF_DIR, "Ahsoka_flat_oracle_standalone"))
+                    if os.path.exists(p)), None)
 B200_CLI = os.path.join(ROOT, "ahsoka_b200", "bin", "Ahsoka_b200")
 
 CASES = [c for c in json.load(open(os.path.join(GOLDEN, "index.json")))["cases"] if "ref_result" in c]
@@ -51,9 +55,9 @@ def _hap_lines(stdout):
 
 @pytest.mark.parametrize("case", CASES, ids=[c["name"] for c in CASES])
 def test_flat_oracle_cli_matches_reference_verbatim(case):
-    exe = os.path.join(REF_DIR, "Ahsoka_flat_oracle")
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/Ahsoka_flat_oracle not built (needs /root/reference at build time)")
+    exe = FLAT_ORACLE
+    if exe is None:
+        pytest.skip("oracle/_ref/Ahsoka_flat_oracle_standalone not built")
     want = open(os.path.join(GOLDEN, case["ref_result"])).read()
     with tempfile.TemporaryDirectory() as td:
         _stage(case, td)
@@ -65,7 +69,7 @@ def test_flat_oracle_cli_matches_reference_verbatim(case):
 def test_reference_verbatim_binary_still_reproduces_golden(case):
     exe = os.path.join(REF_DIR, "Ahsoka_ref")
     if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/Ahsoka_ref not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/Ahsoka_ref not built (needs the original Ahsoka sources at build time: AHSOKA_REFERENCE)")
     want = open(os.path.join(GOLDEN, case["ref_result"])).read()
     with tempfile.TemporaryDirectory() as td:
         _stage(case, td)
@@ -78,14 +82,14 @@ def test_reference_verbatim_binary_still_reproduces_golden(case):
 def test_b200_cli_matches_reference_verbatim(case):
     exe = B200_CLI
     if not os.path.exists(exe):
-        pytest.skip("ahsoka_b200/bin/Ahsoka_b200 not built (needs /root/reference at build time)")
+        pytest.skip("ahsoka_b200/bin/Ahsoka_b200 not built")
     want = open(os.path.join(GOLDEN, case["ref_result"])).read()
     with tempfile.TemporaryDirectory() as td:
         _stage(case, td)
         got, out_gpu = _run_cli(exe, case, td)
         assert got == want
-        ora = os.path.join(REF_DIR, "Ahsoka_flat_oracle")
-        if os.path.exists(ora):
+        ora = FLAT_ORACLE
+        if ora is not None:
             with tempfile.TemporaryDirectory() as td2:
                 _stage(case, td2)
                 _, out_cpu = _run_cli(ora, case, td2)
@@ -117,16 +121,16 @@ def _cfg1_cli(exe):
 
 
 def test_cfg1_flat_oracle_cli_matches_reference_verbatim():
-    exe = os.path.join(REF_DIR, "Ahsoka_flat_oracle")
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/Ahsoka_flat_oracle not built (needs /root/reference at build time)")
+    exe = FLAT_ORACLE
+    if exe is None:
+        pytest.skip("oracle/_ref/Ahsoka_flat_oracle_standalone not built")
     _cfg1_cli(exe)
 
 
 @pytest.mark.gpu
 def test_cfg1_b200_cli_matches_reference_verbatim():
     if not os.path.exists(B200_CLI):
-        pytest.skip("ahsoka_b200/bin/Ahsoka_b200 not built (needs /root/reference at build time)")
+        pytest.skip("ahsoka_b200/bin/Ahsoka_b200 not built")
     _cfg1_cli(B200_CLI)
 
 
@@ -142,9 +146,9 @@ def _readset_dumps(exe, case):
 
 @pytest.mark.parametrize("case", CASES, ids=[c["name"] for c in CASES])
 def test_flat_oracle_cli_readset_final_dumps_match_reference_verbatim(case):
-    ref, exe = os.path.join(REF_DIR, "Ahsoka_ref"), os.path.join(REF_DIR, "Ahsoka_flat_oracle")
-    if not (os.path.exists(ref) and os.path.exists(exe)):
-        pytest.skip("oracle/_ref binaries not built (need /root/reference at build time)")
+    ref, exe = os.path.join(REF_DIR, "Ahsoka_ref"), FLAT_ORACLE
+    if not os.path.exists(ref) or exe is None:
+        pytest.skip("oracle/_ref/Ahsoka_ref not built (needs the original Ahsoka sources at build time: AHSOKA_REFERENCE)")
     want = _readset_dumps(ref, case)
     assert want and _readset_dumps(exe, case) == want
 
@@ -152,9 +156,11 @@ def test_flat_oracle_cli_readset_final_dumps_match_reference_verbatim(case):
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", CASES, ids=[c["name"] for c in CASES])
 def test_b200_cli_readset_final_dumps_match_reference_verbatim(case):
+    # against the original's binary when it was built; else against the drop-in with the CPU oracle behind the C ABI
     ref = os.path.join(REF_DIR, "Ahsoka_ref")
-    if not (os.path.exists(ref) and os.path.exists(B200_CLI)):
-        pytest.skip("binaries not built (need /root/reference at build time)")
+    ref = ref if os.path.exists(ref) else FLAT_ORACLE
+    if ref is None or not os.path.exists(B200_CLI):
+        pytest.skip("binaries not built")
     want = _readset_dumps(ref, case)
     assert want and _readset_dumps(B200_CLI, case) == want
 
@@ -164,7 +170,7 @@ def test_b200_cli_exit_code_tells_when_a_chain_exceeds_a_build_limit():
     # a chain beyond a build limit is reported on stderr, gets header-only output — and the process exits with code 3, so that
     # a dropped chain cannot be mistaken for an empty one (the limit is lowered through the library's testing knob)
     if not os.path.exists(B200_CLI):
-        pytest.skip("ahsoka_b200/bin/Ahsoka_b200 not built (needs /root/reference at build time)")
+        pytest.skip("ahsoka_b200/bin/Ahsoka_b200 not built")
     import sys
     sys.path.insert(0, ROOT)
     from ahsoka_b200 import synth
@@ -178,3 +184,32 @@ def test_b200_cli_exit_code_tells_when_a_chain_exceeds_a_build_limit():
         r = subprocess.run(cmd, cwd=td, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, env=env, timeout=600)
         assert r.returncode == 3 and "NOT phased" in r.stderr
         assert "haplotype 0:" not in open(os.path.join(td, "out-result.txt")).read()
+
+
+def test_standalone_command_line_parser():
+    # the parser a build without the original's sources links (ahsoka_b200/host/standalone/standalone.cpp): the sub-commands
+    # and options of the original's CLI; a wrong command line exits with 1 and says why, -h with 0, an option registered for
+    # another sub-command is ignored, as the original's parser does
+    exe = os.path.join(REF_DIR, "Ahsoka_flat_oracle_standalone")
+    if not os.path.exists(exe):
+        pytest.skip("oracle/_ref/Ahsoka_flat_oracle_standalone not built")
+    case = CASES[0]
+    with tempfile.TemporaryDirectory() as td:
+        _stage(case, td)
+        gfa = os.path.join(GOLDEN, case["gfa"])
+
+        def run(*args):
+            return subprocess.run([exe] + list(args), cwd=td, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600)
+        for args, why in ((["phase", "-g", gfa, "-a", "reads.gaf"], "missing mandatory option -o"),
+                          (["phase", "-g", gfa, "-a", "reads.gaf", "-o", "out", "-z", "1"], "unknown option -z"),
+                          (["phase", "-g", gfa, "-a", "reads.gaf", "-o"], "option -o needs a value"),
+                          (["bogus", "-g", gfa], "unknown sub-command 'bogus'"),
+                          ([], "unknown sub-command ''")):
+            r = run(*args)
+            assert r.returncode == 1 and why in r.stderr and "usage: Ahsoka" in r.stderr, (args, r.returncode, r.stderr[-500:])
+        r = run("phase", "-h")
+        assert r.returncode == 0 and "usage: Ahsoka" in r.stderr
+        r = run("only-bubbles", "-g", gfa, "-o", "bub", "-k", "ignored")
+        assert r.returncode == 0 and os.path.exists(os.path.join(td, "bub-bubbleinfo.txt"))
+        r = run("phase", "-g" + gfa, "-a", "reads.gaf", "-o", "out", "-t", "1")
+        assert r.returncode == 0 and open(os.path.join(td, "out-result.txt")).read() == open(os.path.join(GOLDEN, case["ref_result"])).read()

@@ -2,11 +2,13 @@
 (ahsoka_b200/host/gaf_reader.cpp) and allele-path enumeration (chain_alleles.cpp) against the
 reference's own functions.
 
-oracle/_ref/Ahsoka_flat_oracle links BOTH: the reference translation units alignmentreader.cpp /
-chainstoreadset.cpp compiled where they lie, and this repo's replacements; AHSOKA_HOST=reference
-selects the former.  Everything observable must be byte-identical between the two: the flattened
-batch handed to ahs_phase_batch (AHSOKA_DUMP_BATCH), the <gaf stem>-alignment_identities.txt side
-file, -result.txt, -bubbleinfo.txt and stdout.  Nothing here reads /root/reference at run time.
+oracle/_ref/Ahsoka_flat_oracle (built when AHSOKA_REFERENCE names the original's sources) links BOTH: the
+reference translation units alignmentreader.cpp / chainstoreadset.cpp compiled where they lie, and this repo's
+replacements; AHSOKA_HOST=reference selects the former.  Everything observable must then be byte-identical between
+the two: the flattened batch handed to ahs_phase_batch (AHSOKA_DUMP_BATCH), the <gaf stem>-alignment_identities.txt
+side file, -result.txt, -bubbleinfo.txt and stdout.  Without that binary the same tests run this repo's host stages
+alone (oracle/_ref/Ahsoka_flat_oracle_standalone) and keep every assertion that does not need the original's
+functions: the golden files written by the original, exit codes and messages, determinism.
 """
 import json
 import os
@@ -19,10 +21,20 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-EXE = os.path.join(ROOT, "oracle", "_ref", "Ahsoka_flat_oracle")
+EXE_REF = os.path.join(ROOT, "oracle", "_ref", "Ahsoka_flat_oracle")                    # linked with the original's host stages
+HAS_REF = os.path.exists(EXE_REF)
+EXE = EXE_REF if HAS_REF else os.path.join(ROOT, "oracle", "_ref", "Ahsoka_flat_oracle_standalone")
 CASES = [c for c in json.load(open(os.path.join(GOLDEN, "index.json")))["cases"] if "ref_result" in c]
 
-pytestmark = pytest.mark.skipif(not os.path.exists(EXE), reason="oracle/_ref/Ahsoka_flat_oracle not built (needs /root/reference at build time)")
+pytestmark = pytest.mark.skipif(not os.path.exists(EXE), reason="oracle/_ref/Ahsoka_flat_oracle_standalone not built")
+
+
+def test_reference_checker_is_built_when_the_original_is_given():
+    # a build with AHSOKA_REFERENCE must leave the reference-linked checker: the comparisons below then must not quietly
+    # fall back to this repo's host stages alone
+    if not os.environ.get("AHSOKA_REFERENCE"):
+        pytest.skip("AHSOKA_REFERENCE not set")
+    assert HAS_REF, "AHSOKA_REFERENCE is set but oracle/_ref/Ahsoka_flat_oracle was not built"
 
 
 def _run(td, tag, gfa_text, gaf_bytes, host, ploidy=2, expect_ok=True):
@@ -47,11 +59,13 @@ def _run(td, tag, gfa_text, gaf_bytes, host, ploidy=2, expect_ok=True):
 
 
 def _both(gfa_text, gaf_bytes, ploidy=2):
+    """The native host's outputs, checked against the reference's functions when the checker links them."""
     with tempfile.TemporaryDirectory() as td:
-        ref = _run(td, "ref", gfa_text, gaf_bytes, "reference", ploidy)
         nat = _run(td, "nat", gfa_text, gaf_bytes, "native", ploidy)
-    for k in ref:
-        assert ref[k] == nat[k], "native host differs from the reference's functions in " + k
+        if HAS_REF:
+            ref = _run(td, "ref", gfa_text, gaf_bytes, "reference", ploidy)
+            for k in ref:
+                assert ref[k] == nat[k], "native host differs from the reference's functions in " + k
     return nat
 
 
@@ -135,8 +149,9 @@ def test_unterminated_last_line_is_dropped():
     assert a["reads-alignment_identities.txt"].count(b"\n") == b["reads-alignment_identities.txt"].count(b"\n") + 1
     with tempfile.TemporaryDirectory() as td:      # empty and missing-newline-only files: no alignments, header-only result
         e = _run(td, "empty", gfa, b"", "native")
-        r = _run(td, "empty_ref", gfa, b"", "reference")
-    assert e == r
+        if HAS_REF:
+            assert e == _run(td, "empty_ref", gfa, b"", "reference")
+    assert e["out-result.txt"] and b"haplotype" not in e["out-result.txt"]
 
 
 MALFORMED = {
@@ -159,8 +174,8 @@ def test_malformed_lines_fail_loudly_where_the_reference_dies(kind):
     gaf = b"\n".join(lines) + b"\n"
     with tempfile.TemporaryDirectory() as td:
         nat = _run(td, "nat", gfa, gaf, "native", expect_ok=False)
-        ref = _run(td, "ref", gfa, gaf, "reference", expect_ok=False)
-    assert ref.returncode != 0, "the reference's reader accepted this line"
+        if HAS_REF:
+            assert _run(td, "ref", gfa, gaf, "reference", expect_ok=False).returncode != 0, "the reference's reader accepted this line"
     assert nat.returncode == 65
     assert b"reads.gaf:6:" in nat.stderr
 
@@ -297,6 +312,13 @@ def test_bubble_detection_on_messy_graphs():
     with tempfile.TemporaryDirectory() as td:
         for seed in range(150):
             gfa = _messy_gfa(seed)
+            if not HAS_REF:         # this repo's detection alone: it finishes on every graph and finds the chains it finds with the original
+                nat = _only_bubbles(td, "n%d" % seed, gfa, "native")
+                if nat is not None:
+                    ok += 1
+                    with_bubbles += b"bubble id" in nat[1]
+                    _run(td, "pn%d" % seed, gfa, b"", "native", expect_ok=False)       # terminates (else TimeoutExpired)
+                continue
             ref = _only_bubbles(td, "r%d" % seed, gfa, "reference")
             if ref is None:
                 continue        # the reference itself crashes or does not terminate on this graph
@@ -327,7 +349,8 @@ MALFORMED_GFA = {
 @pytest.mark.parametrize("kind", sorted(MALFORMED_GFA))
 def test_malformed_gfa_fails_loudly_where_the_reference_dies(kind):
     with tempfile.TemporaryDirectory() as td:
-        assert _only_bubbles(td, "ref", MALFORMED_GFA[kind], "reference") is None
+        if HAS_REF:
+            assert _only_bubbles(td, "ref", MALFORMED_GFA[kind], "reference") is None
         d = os.path.join(td, "nat")
         os.makedirs(d)
         open(os.path.join(d, "g.gfa"), "w").write(MALFORMED_GFA[kind])
@@ -378,6 +401,7 @@ def test_reader_thread_count_does_not_change_the_batch():
             assert r.returncode == 0, r.stderr[-2000:]
             outs.append((open(os.path.join(d, "batch.bin"), "rb").read(), open(os.path.join(d, "reads-alignment_identities.txt"), "rb").read(),
                          open(os.path.join(d, "out-result.txt"), "rb").read()))
-        ref = _run(td, "ref", gfa, gaf, "reference")
+        ref = _run(td, "ref", gfa, gaf, "reference") if HAS_REF else None
     assert outs[0] == outs[1] == outs[2]
-    assert outs[0] == (ref["batch.bin"], ref["reads-alignment_identities.txt"], ref["out-result.txt"])
+    if ref is not None:
+        assert outs[0] == (ref["batch.bin"], ref["reads-alignment_identities.txt"], ref["out-result.txt"])
