@@ -43,16 +43,13 @@ struct DB {
     unsigned long long *ch_pairs2;                        // [C] twice the scored pairs of a chain above CC_MAXN reads (k_read_rates): sizes its edge slots
     // ---- final reads (after the host computed the offsets)
     int64_t *frow_off, *pos_off, *code_off, *cw_off;      // [C+1],[C+1],[C],[C]
-    int64_t *cf_off;                                      // [C] offset of a chain's dense cluster-editing workspaces (k_cluster_big: chains of CC_MAXN+1 .. 1024 reads)
     int32_t *fr_chain, *fr_first, *fr_last, *fr_mapq, *fr_id, *fr_nv, *fr_cluster;
     uint32_t *codes;
     int32_t *pos, *pos_compact, *pos_chain;
     // ---- scoring / cluster editing
     uint16_t *es, *ed;
     const int64_t *ln, *ln1;                              // log tables, 1025 entries each
-    int32_t *W; int64_t *F, *P; uint32_t *big_key;        // F, P, big_key: workspaces of k_cluster_big (n x n per chain above CC_MAXN)
-    int32_t *ce_list, *ce_newrow, *ce_label;              // per-node scratch of k_cluster_big: old weights to a / b, merged weight
-    int64_t *ce_rbF, *ce_rbP; int32_t *ce_rbFarg, *ce_rbParg;   //   fresh icf / icp, first / last non-zero column of a row
+    int32_t *W;                                           // pair weights: upper triangle per chain up to CC_MAXN reads, n x n above
     uint64_t *key_scratch; int64_t *key_scratch_off;       // overflow buffers for reads with > 256 partners
     uint8_t *ch_small;                                    // [C] 1 = chain is scored + clustered out of shared memory (k_chain.cuh)
     // ---- consensus / threading

@@ -3,7 +3,7 @@
 // Replaces ReadScoring::scoreReadsetLocal + ClusterEditingSolver::run (call sites reference
 // src/alignmentstoreadset.cpp:308-315; algorithms: oracle/core/phase_core.hpp rules R1 and R2) for
 // chains with at most CC_MAXN final reads — every chain of BASELINE config 2.  Larger chains take
-// the HBM-resident path (k_read_rates / k_pair_scores / k_cluster_big).
+// the HBM-resident path (k_read_rates / k_pair_scores / k_cluster_sparse).
 //
 //   k_score_chain    K2: reads the packed allele rows (code_bytes per cell) + 8 B of row descriptors per
 //                    read, writes one int32 Q10 weight per read pair (upper triangle, row-major): exactly

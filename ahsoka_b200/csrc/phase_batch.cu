@@ -23,7 +23,6 @@
 #include "k_front.cuh"
 #include "k_score.cuh"
 #include "k_chain.cuh"
-#include "k_cluster_big.cuh"
 #include "k_cluster_sparse.cuh"
 #include "host_plan.hpp"
 #include "k_thread.cuh"
@@ -42,7 +41,6 @@ struct ArgFail { std::string msg; };
 struct PassThrough { int rc; std::string msg; };      // failure of one device thread of a multi-device call, re-raised by the caller
 
 constexpr int MAX_READS_CLUSTER = 65535;       // 16-bit node ids in the edge keys of k_cluster_sparse (chains above CC_MAXN reads)
-constexpr int MAX_READS_CLUSTER_DENSE = 8191;  // k_cluster_big (AHS_CLUSTER_BIG=1: the dense predecessor, kept for comparison)
 constexpr int MAX_POSITIONS = 32767;
 constexpr int64_t MAX_READS_CHAIN = (int64_t)1 << 20;        // distinct read names per chain (k_read_rank is quadratic in them)
 constexpr int64_t MAX_BIG_W_BYTES = (int64_t)48 << 30;       // dense weight matrices of the chains above CC_MAXN reads, per call and device
@@ -68,10 +66,11 @@ struct Pool {
 };
 
 // streams and events of one pipeline in flight (a call phases its chains in up to N_LANES chunks, chunk k+1 uploading
-// and projecting while chunk k clusters)
+// and projecting while chunk k clusters).  ev[0..6]: stage boundaries of a pass (collect_times); ev[7], ev[8] of lane 0:
+// the call's own events (DeviceJob)
 struct Lane {
     cudaStream_t stream = nullptr, stream2 = nullptr;
-    cudaEvent_t ev[12], ev_cells = nullptr, ev_en[8], ev_fork = nullptr, ev_join[8], ev_up = nullptr;
+    cudaEvent_t ev[9], ev_cells = nullptr, ev_en[8], ev_fork = nullptr, ev_join[8], ev_up = nullptr;
 };
 constexpr int N_LANES = 4;
 
@@ -100,7 +99,7 @@ struct ScoreClass { int nmax, nt, kpl; };
 static const ScoreClass kScore[] = {{32, 64, 1}, {48, 128, 2}, {64, 128, 2}, {96, 256, 4}, {128, 256, 4}, {160, 256, 8}};
 constexpr int N_SCORE = (int)(sizeof(kScore) / sizeof(kScore[0]));
 
-#define AHS_FOR_EACH_NT(X) X(32, 8) X(64, 8) X(96, 8) X(128, 8) X(192, 8) X(256, 8) X(384, 8) X(512, 8) X(768, 8) X(1024, 8) X(256, 12) X(1024, 9) X(1024, 11) X(1024, 13)
+#define AHS_FOR_EACH_NT(X) X(32, 8) X(64, 8) X(96, 8) X(128, 8) X(192, 8) X(256, 8) X(512, 8) X(768, 8) X(1024, 8) X(256, 12) X(1024, 9) X(1024, 11) X(1024, 13)
 #define AHS_FOR_EACH_SC(X) X(64, 1) X(128, 2) X(256, 4) X(256, 8)
 static void chain_kernel_attributes(size_t optin) {
 #define X(NT, PER) CK(cudaFuncSetAttribute(k_cluster_chain<NT, PER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)optin)); \
@@ -222,7 +221,6 @@ static Ctx* get_ctx(int device) {
     build_canon_tables(c->canon);
     c->smem_optin = prop.sharedMemPerBlockOptin;
     check_classes(c->smem_optin);
-    CK(cudaFuncSetAttribute(k_cluster_big, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
     CK(cudaFuncSetAttribute(k_cluster_sparse<SP_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
     CK(cudaFuncSetAttribute(k_cluster_sparse<SP_THREADS_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
     chain_kernel_attributes(c->smem_optin);
@@ -287,7 +285,6 @@ struct Pipeline {
     int64_t* h_sc = nullptr;                                                   // pinned scalars of sync #1: cells, error flags, largest allele count
     unsigned long long* h_cells = nullptr;
     char *sg_h = nullptr, *sg_d = nullptr; size_t sg_cap = 0;                   // pinned / device staging block of phase 2
-    float ms_smem_cluster = 0;
     bool early_out = false;                                                     // download the matrix while the clustering runs
     int64_t base_allele = 0, base_anode = 0, base_enode = 0;                    // first elements of the three big offset arrays (chunk views)
     int64_t cell_base = 0;                                                      // cells of the chunks before this one (cell_off is global)
@@ -295,7 +292,7 @@ struct Pipeline {
     int64_t n_code_words = 0, n_cw = 0, h_tot_cells = 0, h_slots = 0;
     size_t front_smem = 0; bool use_front = false;                              // one block per chain for projection + rows (k_front.cuh)
     std::vector<uint32_t> front_need;                                           // per chain: shared memory of its block
-    float ms[8] = {0};
+    float ms[7] = {0};
     int n_launches = 0;
 
     template <class T> const T* up(const T* h, int64_t n) {
@@ -373,7 +370,7 @@ struct Pipeline {
                 else { front_need[c] = fr_layout((int)B, (int)R, (int)nal, (int)NEc, (int)NENc, (int)cap).total; front_smem = std::max(front_smem, (size_t)front_need[c]); }
             }
         }
-        use_front = front_smem <= FR_SMEM_CAP && getenv("AHS_NO_FRONT") == nullptr;
+        use_front = front_smem <= FR_SMEM_CAP;
         d.hoff = up_pinned(hoff.data(), C); d.hmaskc = up_pinned(hmaskc.data(), C);
         CK(cudaStreamWaitEvent(st, ln->ev_en[N_EN - 1], 0));
         CK(cudaEventRecord(ln->ev_up, st));                    // the copies are through: the next range's may start
@@ -404,7 +401,7 @@ struct Pipeline {
         d.ln = cx->d_ln; d.ln1 = cx->d_ln1;
         h_status = cx->pin.get<int32_t>(C); h_nfinal = cx->pin.get<int32_t>(C); h_npos = cx->pin.get<int32_t>(C); h_sc = cx->pin.get<int64_t>(4);
         h_cells = cx->pin.get<unsigned long long>(C);
-        sg_cap = (size_t)(C + 2) * (8 * 6 + 4 * 3 + 1) + 512;
+        sg_cap = (size_t)(C + 2) * (8 * 5 + 4 * 3 + 1) + 512;
         sg_h = (char*)cx->pin.alloc(sg_cap); sg_d = (char*)cx->dev.alloc(sg_cap);
     }
 
@@ -534,10 +531,9 @@ struct Pipeline {
         if (in->ploidy > 4) S_max = cn_count(in->ploidy, in->ploidy + 2);      // canonical tuples over p + 2 clusters (rule R3c)
         d.S_max = (int32_t)S_max;
         Stage sg; sg.h = sg_h; sg.dv = sg_d;
-        int64_t *dv_frow, *dv_pos, *dv_code, *dv_cw, *dv_back, *dv_cf; int32_t *dv_words, *dv_order, *dv_status; uint8_t* dv_small;
+        int64_t *dv_frow, *dv_pos, *dv_code, *dv_cw, *dv_back; int32_t *dv_words, *dv_order, *dv_status; uint8_t* dv_small;
         int64_t* s_frow = sg.take<int64_t>(C + 1, &dv_frow); int64_t* s_pos = sg.take<int64_t>(C + 1, &dv_pos);
         int64_t* s_code = sg.take<int64_t>(C, &dv_code); int64_t* s_cw = sg.take<int64_t>(C, &dv_cw); int64_t* s_back = sg.take<int64_t>(C, &dv_back);
-        int64_t* s_cf = sg.take<int64_t>(C, &dv_cf); int64_t n_cf = 0;
         int32_t* s_words = sg.take<int32_t>(C, &dv_words); int32_t* s_order = sg.take<int32_t>(C, &dv_order); int32_t* s_status = sg.take<int32_t>(C, &dv_status);
         uint8_t* s_small = sg.take<uint8_t>(C, &dv_small);
         if (sg.used > sg_cap) throw std::runtime_error("staging block overflow");
@@ -545,13 +541,9 @@ struct Pipeline {
         bool status_changed = false;
         s_frow[0] = 0; s_pos[0] = 0;
         int64_t nf_big = 0, cells_ok = 0; int n_max = 0;
-        // chains above CC_MAXN reads: dense workspaces (k_cluster_big) up to dense_max reads, edge slots + lists (k_cluster_sparse) above
-        // chains above CC_MAXN reads take k_cluster_sparse (edge slots + lists).  AHS_CLUSTER_BIG=1 (comparison runs): its dense
-        // predecessor k_cluster_big up to 8,191 reads — slower since the sparse kernel balances its warps (cfg4 x 0.5: 599 vs 545 ms)
-        const int dense_max = (getenv("AHS_CLUSTER_BIG") && atoi(getenv("AHS_CLUSTER_BIG"))) ? MAX_READS_CLUSTER_DENSE : CC_MAXN;
-        const int sp_small_n = getenv("AHS_SP_SMALL_N") ? atoi(getenv("AHS_SP_SMALL_N")) : SP_SMALL_N;
+        // chains above CC_MAXN reads take k_cluster_sparse (edge slots + lists)
         int max_reads = MAX_READS_CLUSTER;
-        int64_t nf_dense = 0, nf_sparse = 0;
+        int64_t nf_sparse = 0;
         if (const char* e = getenv("AHS_MAX_READS_CLUSTER")) max_reads = std::max(CC_MAXN, std::min(max_reads, atoi(e)));      // tests: exercise the limit cheaply
         int64_t big_w_bytes = 0;
         for (int64_t c = 0; c < C; c++) {
@@ -571,8 +563,7 @@ struct Pipeline {
             s_code[c] = n_code_words; n_code_words += n * s_words[c];
             s_small[c] = (n > 0 && n <= CC_MAXN) ? 1 : 0;
             s_cw[c] = n_cw; n_cw += s_small[c] ? n * (n - 1) / 2 : n * n;
-            s_cf[c] = n_cf;
-            if (n > CC_MAXN && n <= dense_max) { n_cf += n * n; nf_dense += n; } else if (n > dense_max) nf_sparse += n;
+            if (n > CC_MAXN) nf_sparse += n;
             s_back[c] = s_pos[c] * S_max;
             if (!s_small[c]) nf_big += n;
             n_max = std::max<int>(n_max, (int)n);
@@ -596,7 +587,7 @@ struct Pipeline {
         // bulk upload of the next range
         { const int64_t n16 = (int64_t)((sg.used + 15) / 16); k_fetch_host<<<grid_for(n16, 256, sms), 256, 0, st>>>((const int4*)sg.h, (int4*)sg.dv, n16); n_launches += 1; }
         d.frow_off = dv_frow; d.pos_off = dv_pos; d.code_off = dv_code; d.cw_off = dv_cw; d.back_off = dv_back;
-        d.ch_words = dv_words; d.ch_small = dv_small; d.cf_off = dv_cf;
+        d.ch_words = dv_words; d.ch_small = dv_small;
         if (status_changed) CK(cudaMemcpyAsync(d.ch_status, dv_status, C * 4, cudaMemcpyDeviceToDevice, st));
         d.fr_chain = dalloc<int32_t>(NF); d.fr_first = dalloc<int32_t>(NF); d.fr_last = dalloc<int32_t>(NF); d.fr_mapq = dalloc<int32_t>(NF);
         d.fr_id = dalloc<int32_t>(NF); d.fr_nv = dalloc<int32_t>(NF); d.fr_cluster = dzero<int32_t>(NF);
@@ -605,14 +596,9 @@ struct Pipeline {
         d.es = dalloc<uint16_t>(NF); d.ed = dalloc<uint16_t>(NF);
         d.W = dalloc<int32_t>(n_cw);
         if (nf_big) {
-            // HBM-resident path (chains above CC_MAXN reads): dense n x n workspaces
+            // HBM-resident path (chains above CC_MAXN reads): a dense n x n weight matrix per chain
             for (int64_t c = 0; c < C; c++) if (!s_small[c] && h_nfinal[c] > 0)
                 CK(cudaMemsetAsync(d.W + s_cw[c], 0, (size_t)h_nfinal[c] * h_nfinal[c] * 4, st));
-            if (nf_dense) {
-                d.F = dalloc<int64_t>(n_cf); d.P = dalloc<int64_t>(n_cf); d.big_key = dalloc<uint32_t>(n_cf);
-                d.ce_list = dalloc<int32_t>(NF); d.ce_newrow = dalloc<int32_t>(NF);
-                d.ce_label = dalloc<int32_t>(NF); d.ce_rbF = dalloc<int64_t>(NF); d.ce_rbP = dalloc<int64_t>(NF); d.ce_rbFarg = dalloc<int32_t>(NF); d.ce_rbParg = dalloc<int32_t>(NF);
-            }
         }
         d.rec = dalloc<PosRec>(NP); d.back = dalloc<uint16_t>(NP * S_max);
         d.path = dzero<int32_t>(NP * in->ploidy); d.hap_allele = dzero<uint8_t>(NP * in->ploidy); d.dp_cost = dzero<double>(C);
@@ -654,7 +640,7 @@ struct Pipeline {
             CK(cudaStreamSynchronize(st));
             std::vector<SpChain> chs;
             int64_t slots = 0, pool = 0, nodes = 0, leaves = 0, sups = 0;
-            int firstb, lenb; range_of(dense_max + 1, MAX_READS_CLUSTER, firstb, lenb);
+            int firstb, lenb; range_of(CC_MAXN + 1, MAX_READS_CLUSTER, firstb, lenb);
             for (int k = 0; k < lenb; k++) {
                 const int c = s_order[firstb + k];
                 SpChain ch{};
@@ -666,7 +652,7 @@ struct Pipeline {
                 ch.node_off = nodes; ch.leaf_off = leaves; ch.sup_off = sups;
                 slots += e0; pool += ch.list_cap; nodes += ch.n; leaves += ch.n_leaf; sups += ch.n_sup;
                 sp_nmax = std::max(sp_nmax, ch.n); sp_max_leaf = std::max(sp_max_leaf, ch.n_leaf);
-                if (ch.n > sp_small_n) sp_n_large++;                               // the list is sorted by decreasing read count
+                if (ch.n > SP_SMALL_N) sp_n_large++;                               // the list is sorted by decreasing read count
                 else { sp_nmax_small = std::max(sp_nmax_small, ch.n); sp_leaf_small = std::max(sp_leaf_small, ch.n_leaf); }
                 chs.push_back(ch);
             }
@@ -704,7 +690,6 @@ struct Pipeline {
         for (int i = 0; i < 8; i++) { CK(cudaEventRecord(ln->ev_join[i], cx->side[i])); CK(cudaStreamWaitEvent(st, ln->ev_join[i], 0)); }
         CK(cudaEventRecord(ln->ev[3], st));
         // ---- cluster editing out of shared memory
-        CK(cudaEventRecord(ln->ev[10], st));
         // the size classes run on four side streams so that the tail of one class overlaps the bulk of the next
         CK(cudaEventRecord(ln->ev_fork, st));
         for (auto& t : cx->side) CK(cudaStreamWaitEvent(t, ln->ev_fork, 0));
@@ -719,31 +704,21 @@ struct Pipeline {
             cluster_launch(nt, kCluster[k].per, grid, smem, cx->side[q++ & 7], d, dv_order + first, len, kCluster[k].nmax, counters + 8 + N_SCORE + k, scratch); n_launches += 1;
         }
         // ---- cluster editing of the chains above CC_MAXN reads, on two of the side streams (next to the shared-memory classes)
-        if (nf_big) {
-            int first, len; range_of(CC_MAXN + 1, dense_max, first, len);
-            if (len) {
-                const size_t sm_big = cb_smem_bytes(std::min<int>(n_max, dense_max));
-                const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / (sm_big + 1024)));
-                k_cluster_big<<<(unsigned)std::min<int64_t>(len, (int64_t)sms * per_sm), CB_THREADS, sm_big, cx->side[5]>>>(d, dv_order + first, len, std::min<int>(n_max, dense_max), counters + 4);
+        if (sp.n_chains) {
+            // the few long chains in blocks of 1024 threads, the many short ones (<= 1024 reads) 256 threads each, several per SM:
+            // a greedy step is a chain of dependent memory latencies, which only other chains can hide
+            if (sp_n_large) {
+                k_cluster_sparse<SP_THREADS><<<(unsigned)std::min<int64_t>(sp_n_large, sms), SP_THREADS, sp_smem_bytes(sp_nmax, sp_max_leaf), cx->side[7]>>>(d, sp, 0, sp_n_large, sp_nmax, sp_max_leaf, counters + 2);
                 n_launches += 1;
             }
-            if (sp.n_chains) {
-                // the few long chains in blocks of 1024 threads, the many short ones (<= 1024 reads) 256 threads each, several per SM:
-                // a greedy step is a chain of dependent memory latencies, which only other chains can hide
-                if (sp_n_large) {
-                    k_cluster_sparse<SP_THREADS><<<(unsigned)std::min<int64_t>(sp_n_large, sms), SP_THREADS, sp_smem_bytes(sp_nmax, sp_max_leaf), cx->side[7]>>>(d, sp, 0, sp_n_large, sp_nmax, sp_max_leaf, counters + 2);
-                    n_launches += 1;
-                }
-                if (sp.n_chains > sp_n_large) {
-                    const size_t sm_small = sp_smem_bytes(sp_nmax_small, sp_leaf_small);
-                    const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / (sm_small + 1024)));
-                    k_cluster_sparse<SP_THREADS_SMALL><<<(unsigned)std::min<int64_t>(sp.n_chains - sp_n_large, (int64_t)sms * per_sm), SP_THREADS_SMALL, sm_small, cx->side[6]>>>(d, sp, sp_n_large, sp.n_chains, sp_nmax_small, sp_leaf_small, counters + 3);
-                    n_launches += 1;
-                }
+            if (sp.n_chains > sp_n_large) {
+                const size_t sm_small = sp_smem_bytes(sp_nmax_small, sp_leaf_small);
+                const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / (sm_small + 1024)));
+                k_cluster_sparse<SP_THREADS_SMALL><<<(unsigned)std::min<int64_t>(sp.n_chains - sp_n_large, (int64_t)sms * per_sm), SP_THREADS_SMALL, sm_small, cx->side[6]>>>(d, sp, sp_n_large, sp.n_chains, sp_nmax_small, sp_leaf_small, counters + 3);
+                n_launches += 1;
             }
         }
         for (int i = 0; i < 8; i++) { CK(cudaEventRecord(ln->ev_join[i], cx->side[i])); CK(cudaStreamWaitEvent(st, ln->ev_join[i], 0)); }
-        CK(cudaEventRecord(ln->ev[11], st));
         CK(cudaEventRecord(ln->ev[4], st));
         // ---- coverage / consensus, threading
         if (NP && BITS == 2) { k_consensus_chain<<<grid_for(C, 4, sms), 128, 0, st>>>(d); n_launches += 1; }      // chains with <= 16 clusters
@@ -756,7 +731,6 @@ struct Pipeline {
         else if (NP && in->ploidy <= 4) { k_thread<<<std::min<int64_t>(C, (int64_t)sms * 8), DP_THREADS, 21 * (size_t)S_max + 64, st>>>(d, counters + 1); n_launches += 1; }
         else if (NP) { k_thread_canon<<<std::min<int64_t>(C, (int64_t)sms * 4), CN_THREADS, 64 * 1024, st>>>(d, cx->canon, counters + 1); n_launches += 1; }
         CK(cudaEventRecord(ln->ev[6], st));
-        CK(cudaEventRecord(ln->ev[7], st));
         CK(cudaGetLastError());
     }
 
@@ -769,10 +743,9 @@ struct Pipeline {
         CK(cudaEventElapsedTime(&t, ln->ev[1], ln->ev[2])); ms[1] = t;
         CK(cudaEventElapsedTime(&t, ln->ev[2], ln->ev[3])); ms[2] = t;
         CK(cudaEventElapsedTime(&t, ln->ev[3], ln->ev[4])); ms[3] = t;
-        CK(cudaEventElapsedTime(&t, ln->ev[10], ln->ev[11])); ms_smem_cluster = t; ms[7] = t;      // shared-memory cluster editing alone
         CK(cudaEventElapsedTime(&t, ln->ev[4], ln->ev[5])); ms[4] = t;
         CK(cudaEventElapsedTime(&t, ln->ev[5], ln->ev[6])); ms[5] = t;
-        CK(cudaEventElapsedTime(&t, ln->ev[0], ln->ev[7])); ms[6] = t;
+        CK(cudaEventElapsedTime(&t, ln->ev[0], ln->ev[6])); ms[6] = t;
     }
 
     // where this pipeline's results go inside the arrays of ahs_batch_out (a chunk writes a slice)
@@ -883,7 +856,7 @@ struct DeviceJob {
     std::vector<ChainView> views; std::vector<Pipeline> pls; std::vector<Sizes> szs;
     std::unique_lock<std::mutex> lock;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
-    float acc[8] = {0}, h2d = 0, d2h = 0;
+    float acc[7] = {0}, h2d = 0, d2h = 0;
     int iters = 0; int64_t* h_pairs = nullptr;
     HostTrace tr;
 
@@ -903,7 +876,7 @@ struct DeviceJob {
         iters = iters_;
         const int n = (int)ranges.size();
         views.resize(n); pls.resize(n); szs.resize(n);
-        e0 = cx->lanes[0].ev[8]; e1 = cx->lanes[0].ev[9];
+        e0 = cx->lanes[0].ev[7]; e1 = cx->lanes[0].ev[8];
         CK(cudaSetDevice(device));
         CK(cudaEventRecord(e0, cx->lanes[0].stream));
         bool first = true; Lane* last_up = nullptr;
@@ -935,7 +908,7 @@ struct DeviceJob {
                     pl.run();
                     CK(cudaStreamSynchronize(pl.ln->stream));
                     pl.collect_times();
-                    if (it >= warmup) for (int i = 0; i < 8; i++) acc[i] += pl.ms[i];
+                    if (it >= warmup) for (int i = 0; i < 7; i++) acc[i] += pl.ms[i];
                 }
                 if (k + 1 < n) prepare(k + 1);
                 continue;
@@ -955,7 +928,7 @@ struct DeviceJob {
         CK(cudaSetDevice(device));
         h_pairs = cx->pin.get<int64_t>(std::max(n, 1));
         CK(cudaEventSynchronize(e1)); CK(cudaEventElapsedTime(&h2d, e0, e1));
-        cudaEvent_t d0 = cx->lanes[0].ev[8];
+        cudaEvent_t d0 = cx->lanes[0].ev[7];
         CK(cudaEventRecord(d0, cx->lanes[0].stream2));
         for (int k = 0; k < n; k++) {
             h_pairs[k] = 0;
@@ -985,24 +958,24 @@ struct DeviceJob {
     }
 
     // stage times of this device: summed over its ranges (resident mode: averaged over the timed iterations)
-    void times(float* ms8, int& launches) {
+    void times(float* ms7, int& launches) {
         const int n = (int)ranges.size();
-        for (int i = 0; i < 8; i++) ms8[i] = 0;
+        for (int i = 0; i < 7; i++) ms7[i] = 0;
         launches = 0;
-        if (iters > 0) { for (int i = 0; i < 8; i++) ms8[i] = acc[i] / iters; for (auto& pl : pls) launches += pl.n_launches; return; }
+        if (iters > 0) { for (int i = 0; i < 7; i++) ms7[i] = acc[i] / iters; for (auto& pl : pls) launches += pl.n_launches; return; }
         int firstk = -1, last = -1;
         for (int k = 0; k < n; k++) if (szs[k].C) {
-            if (n <= N_LANES) { pls[k].collect_times(); for (int i = 0; i < 6; i++) ms8[i] += pls[k].ms[i]; }      // a lane's events are re-recorded by a later range
+            if (n <= N_LANES) { pls[k].collect_times(); for (int i = 0; i < 6; i++) ms7[i] += pls[k].ms[i]; }      // a lane's events are re-recorded by a later range
             launches += pls[k].n_launches;
             if (firstk < 0) firstk = k; last = k;
         }
-        if (firstk >= 0 && n <= N_LANES) { float t = 0; CK(cudaEventElapsedTime(&t, pls[firstk].ln->ev[0], pls[last].ln->ev[7])); ms8[6] = t; }      // first kernel -> last kernel
+        if (firstk >= 0 && n <= N_LANES) { float t = 0; CK(cudaEventElapsedTime(&t, pls[firstk].ln->ev[0], pls[last].ln->ev[6])); ms7[6] = t; }      // first kernel -> last kernel
         if (getenv("AHS_TRACE") && n <= N_LANES)          // device timeline of the ranges, ms after the call's first event
             for (int k = 0; k < n; k++) if (szs[k].C) {
                 auto at = [&](cudaEvent_t e) { float t = 0; CK(cudaEventElapsedTime(&t, e0, e)); return t; };
                 Lane* l = pls[k].ln;
-                fprintf(stderr, "[ahs timeline] dev %d range %d chains %lld: uploaded %.2f | phase1 start %.2f front %.2f rows+sync1 %.2f score %.2f cluster %.2f consensus %.2f thread %.2f end %.2f\n",
-                        device, k, (long long)szs[k].C, at(l->ev_up), at(l->ev[0]), at(l->ev[1]), at(l->ev[2]), at(l->ev[3]), at(l->ev[4]), at(l->ev[5]), at(l->ev[6]), at(l->ev[7]));
+                fprintf(stderr, "[ahs timeline] dev %d range %d chains %lld: uploaded %.2f | phase1 start %.2f front %.2f rows+sync1 %.2f score %.2f cluster %.2f consensus %.2f thread %.2f\n",
+                        device, k, (long long)szs[k].C, at(l->ev_up), at(l->ev[0]), at(l->ev[1]), at(l->ev[2]), at(l->ev[3]), at(l->ev[4]), at(l->ev[5]), at(l->ev[6]));
             }
     }
 };
@@ -1164,13 +1137,13 @@ static void phase_on_devices(const ahs_batch_in* in, ahs_batch_out* out, const i
     // ---- timings (max over devices) and byte counts
     int bits = 2;
     for (int g = 0; g < G; g++) {
-        float ms8[8]; int launches = 0;
+        float ms7[7]; int launches = 0;
         CK(cudaSetDevice(devs[g]));
-        jobs[g].times(ms8, launches);
+        jobs[g].times(ms7, launches);
         out->ms_h2d = std::max(out->ms_h2d, jobs[g].h2d); out->ms_d2h = std::max(out->ms_d2h, jobs[g].d2h);
-        out->ms_project = std::max(out->ms_project, ms8[0]); out->ms_rows = std::max(out->ms_rows, ms8[1]); out->ms_score = std::max(out->ms_score, ms8[2]);
-        out->ms_cluster = std::max(out->ms_cluster, ms8[3]); out->ms_consensus = std::max(out->ms_consensus, ms8[4]); out->ms_thread = std::max(out->ms_thread, ms8[5]);
-        out->ms_total_device = std::max(out->ms_total_device, ms8[6]);
+        out->ms_project = std::max(out->ms_project, ms7[0]); out->ms_rows = std::max(out->ms_rows, ms7[1]); out->ms_score = std::max(out->ms_score, ms7[2]);
+        out->ms_cluster = std::max(out->ms_cluster, ms7[3]); out->ms_consensus = std::max(out->ms_consensus, ms7[4]); out->ms_thread = std::max(out->ms_thread, ms7[5]);
+        out->ms_total_device = std::max(out->ms_total_device, ms7[6]);
         out->n_launches += launches;
         for (auto& pl : jobs[g].pls) if (pl.sz.C) bits = std::max(bits, (int)pl.d.bits);
     }
@@ -1206,7 +1179,9 @@ double ahs_chain_cost(int64_t n_bubbles, int64_t n_entries, int64_t n_entry_node
     // SM-milliseconds of one chain, calibrated on B200 from the per-class launch times of cfg2 and the stage times of the other
     // configurations (DESIGN.md section 8).  nf = final reads ~ 0.7 x entries.  Projection / rows / scoring / consensus stream
     // the alignment nodes; cluster editing dominates: ~nf^2 in the shared-memory kernel (its parallel width grows with the
-    // pairs), ~nf^3 in the dense big-chain kernel, ~nf x neighbourhood in the sparse one; the threading DP is per position x states.
+    // pairs), ~nf^3 up to 1,024 reads, ~nf x neighbourhood above; the threading DP is per position x states.  The nf^3 regime
+    // predates k_cluster_sparse, which now takes every chain above CC_MAXN reads: it was calibrated on that kernel's dense
+    // predecessor and is kept as it is, because it sets the range count (ranges_of_share) and the device cuts (plan_devices).
     const double nf = 0.7 * (double)n_entries;
     double cluster;
     if (nf <= 160.0) cluster = 2.9e-5 * nf * nf;

@@ -230,13 +230,9 @@ def test_std_sort_replay_including_the_heap_sort_fallback(desc):
             assert np.array_equal(gk, wk) and np.array_equal(gv, wv), (n, desc)
 
 
-@pytest.mark.parametrize("kernel", ["sparse", "dense"])
-def test_cfg4_shape_tetraploid_chains_of_200_to_330_reads(kernel, monkeypatch):
+def test_cfg4_shape_tetraploid_chains_of_200_to_330_reads():
     # BASELINE configs[3] at its shape: ploidy 4, 60x -> 200-330 final reads per chain: HBM-resident scoring, the
-    # big-chain cluster editing and the 4096-state threading DP together.  Chains above 160 reads take k_cluster_sparse;
-    # "dense" selects its predecessor k_cluster_big (kept for comparison runs) on the same input
-    if kernel == "dense":
-        monkeypatch.setenv("AHS_CLUSTER_BIG", "1")
+    # big-chain cluster editing (k_cluster_sparse, chains above 160 reads) and the 4096-state threading DP together
     b = synth.generate(synth.config("cfg4", 0.005))
     got = _check(b)
     assert b.ploidy == 4 and got.n_chains_ok == b.n_chains

@@ -1,5 +1,6 @@
-"""Reads-per-chain histogram of a workload after filtering, and how the chains split between the shared-memory
-cluster-editing kernel (<= 128 reads) and k_cluster_big.  python tools/big_stats.py --workload cfg3 --scale 0.25"""
+"""Reads-per-chain histogram of a workload after filtering, in bands of final reads per chain with each band's share of
+sum n^3 (chains of up to 160 reads cluster in shared memory, longer ones in k_cluster_sparse).
+python tools/big_stats.py --workload cfg3 --scale 0.25"""
 import argparse
 import os
 import sys

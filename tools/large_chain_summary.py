@@ -7,8 +7,7 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 tag = sys.argv[1]
 G, P = os.path.join(ROOT, "gpurun_out"), os.path.join(ROOT, "profiles")
-CASES = [("cfg4 x 0.05 (500 chains of 200-330 reads), default route", f"{tag}_cfg4_sparse_raw.csv"),
-         ("cfg4 x 0.05, AHS_CLUSTER_BIG=1 (the dense predecessor)", f"{tag}_cfg4_big_raw.csv"),
+CASES = [("cfg4 x 0.05 (500 chains of 200-330 reads)", f"{tag}_cfg4_sparse_raw.csv"),
          ("cfg1 (one chain of 1,400 reads)", f"{tag}_cfg1_sparse_raw.csv")]
 
 
