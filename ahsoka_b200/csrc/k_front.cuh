@@ -1,16 +1,15 @@
-// k_front.cuh — projection, stage A, boundary set, stage B, filter and read order of ONE CHAIN PER BLOCK, out of shared memory.
+// k_front.cuh — the front end (projection, stage A, boundary set, stage B, filter, read order) of ONE CHAIN PER BLOCK, out of
+// shared memory.
 //
-// Replaces, for batches whose chains fit (every chain of BASELINE configs 2-4), the kernel sequence k_owner x4,
-// k_validate_owned, k_rank_a, k_validate_perm, k_build_triggers, k_project, k_read_stage_a, k_chain_flags, k_chain_T,
-// k_read_rows, k_read_rank, k_chain_sort, k_count_pos of k_project.cuh — same statements, same results (reference
-// src/alignmentstoreadset.cpp:90-136 stage A, :146-209 filter + boundary set, :210-254 stage B, :262-297 filter +
-// ReadSet::sort(), is_subset :495-548) — with the chain's working set held on chip:
-//   * the chain's slice of the alignment nodes (3/4 of the batch's bytes; entries of a chain are contiguous) arrives by ONE
-//     bulk asynchronous copy (cp.async.bulk + mbarrier) while the block builds the chain's trigger table;
-//   * the read x bubble mask (u16 per cell) lives in shared memory: the projection's atomicOr, the stage-A scan, the stage-B
-//     rewrite into allele codes all stay on chip, and the matrix crosses HBM once, as final codes (k_project.cuh's path
-//     moves ~9x the matrix: memset, atomics, two scans, a rewrite);
-//   * chain-level reductions (maxpos, boundary flags, read counts) are block barriers instead of kernel boundaries.
+// For batches whose chains fit (every chain of BASELINE configs 2-4) it replaces the kernel sequence of k_project.cuh and
+// calls the same rule functions.  What differs is where the data lives and how the work is dealt out:
+//   * ids are chain-local (an allele finds its bubble by binary search: no owner maps);
+//   * the chain's slice of the alignment nodes (3/4 of the batch's bytes) arrives by ONE bulk asynchronous copy
+//     (cp.async.bulk + mbarrier) while the block builds the chain's trigger table;
+//   * the mask and every per-read and per-bubble array live in shared memory, and the matrix crosses HBM once, as final
+//     codes (the sequence moves ~9x the matrix: memset, atomics, two scans, a rewrite);
+//   * chain-level values are scal[] words and block barriers instead of d.ch_* arrays and kernel boundaries;
+//   * thread 0 sorts the read order while the other warps write the results out.
 #pragma once
 #include "common.cuh"
 #include "device_batch.cuh"
@@ -42,12 +41,6 @@ __host__ __device__ inline FrLayout fr_layout(int B, int R, int NA, int NE, int 
 }
 
 __device__ __forceinline__ uint32_t fr_smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-// is value q among the L nodes of the entry (in shared memory)?  (whole lane group)
-__device__ __forceinline__ bool fr_entry_has(const int32_t* nodes, int L, int32_t q, int gl, unsigned gm) {
-    bool f = false;
-    for (int x = gl; x < L; x += FR_G) f |= nodes[x] == q;
-    return __any_sync(gm, f);
-}
 
 // scal[]: 0 maxpos 1 flags 2 T 3 nfinal 4 status 5 npos 6,7 cells (u64) 8 work item 9 err
 // chains [c_begin, c_end): one launch per range of chains with a similar shared-memory need (the chains arrive largest first)
@@ -101,6 +94,7 @@ __global__ void __launch_bounds__(FR_THREADS, 5) k_chain_front(DB d, int c_begin
         int4* rd = (int4*)(fr_sm + L.rd);                                // {nv, first, last, mapq}
         uint8_t* pass = fr_sm + L.pass; int32_t* ord = (int32_t*)(fr_sm + L.ord); int32_t* okey = (int32_t*)(fr_sm + L.okey);
         int32_t* scal = (int32_t*)(fr_sm + L.scal);
+        const float* ident = d.entry_identity + e0;
         // ---- S0: the chain's alignment nodes by one bulk copy; everything else initialised meanwhile
         const int lead = (int)(en0 & 3);                                // the copy starts at the 16-byte boundary below the slice
         if (tid == 0 && NEN > 0) {
@@ -118,104 +112,35 @@ __global__ void __launch_bounds__(FR_THREADS, 5) k_chain_front(DB d, int c_begin
         for (int r = tid; r < R; r += FR_THREADS) { ckey[r] = KEY_NONE; ckeyA[r] = KEY_NONE; fent[r] = 0xffffffffu; good_r[r] = 0; pass[r] = 0; }
         if (tid < 16) scal[tid] = tid == 0 ? -1 : 0;
         __syncthreads();
-        // stage-A visit rank of each bubble (inverse of stage_a_order, :90); a value out of range or twice = not a permutation
-        for (int ob = tid; ob < B; ob += FR_THREADS) {
-            if (d.stage_a_order) { const int32_t v = d.stage_a_order[b0g + ob]; if (v < 0 || v >= B) scal[9] = 16; else rankA[v] = ob; }
-            else rankA[ob] = B - 1 - ob;
+        // stage-A visit ranks and the input checks of the sequence's k_validate_owned / k_rank_a / k_validate_perm
+        {
+            const int32_t* order = d.stage_a_order ? d.stage_a_order + b0g : nullptr;
+            for (int ob = tid; ob < B; ob += FR_THREADS) if (!rank_a_store(rankA, order, ob, B)) scal[9] = 16;
         }
-        for (int e = tid; e < NE; e += FR_THREADS) { const int32_t r = d.entry_read[e0 + e]; if (r < 0 || r >= R) scal[9] = 8; }
+        for (int e = tid; e < NE; e += FR_THREADS) if (!entry_read_ok(d.entry_read[e0 + e], R)) scal[9] = 8;
         __syncthreads();
         for (int b = tid; b < B; b += FR_THREADS) if (rankA[b] < 0) scal[9] = 16;
         __syncthreads();
         if (scal[9]) { if (tid == 0) atomicOr(d.err_flags, scal[9]); if (NEN > 0) { while (true) { uint32_t ok; asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }" : "=r"(ok) : "r"(fr_smem_addr(&s_bar)), "r"(bar_phase) : "memory"); if (ok) break; } bar_phase ^= 1; } continue; }
-        // ---- S1: trigger table of the chain (k_build_triggers)
+        // ---- S1: trigger table of the chain
         for (int ga = tid; ga < NA; ga += FR_THREADS) {
             int lo = 0, hi = B - 1;                                     // bubble of the allele
             while (lo < hi) { const int mid = (lo + hi) >> 1; if (aoff[mid + 1] > ga) hi = mid; else lo = mid + 1; }
-            const int b = lo, a = ga - aoff[b];
             const int64_t o = d.anode_off[a0 + ga];
-            const int len = (int)(d.anode_off[a0 + ga + 1] - o);
-            inc[ga] = -1;
-            arec[ga] = make_int4((int)((uint32_t)b | ((uint32_t)a << 20) | (len == 3 ? 0x80000000u : 0u)), len == 3 ? d.anode[o] : 0, len == 3 ? d.anode[o + 2] : 0, rankA[b]);
-            if (len <= 2) { atomicMin(&univ[b], (uint32_t)a); atomicOr(&scal[1], CH_HAS_UNIV); }      // no inner node: matches every entry (A#9)
-            const uint32_t trig = (uint32_t)(len >= 3 ? d.anode[o + 1] : d.anode[o]);
-            uint32_t slot = hash_slot(trig, hmask);
-            while (true) {
-                const unsigned long long claimed = (0xfffffffeull << 32) | trig;          // head = -2: no allele linked yet
-                const unsigned long long prev = atomicCAS(&tab[slot], SLOT_EMPTY, claimed);
-                if (prev == SLOT_EMPTY || (uint32_t)prev == trig) break;
-                slot = (slot + 1) & hmask;
-            }
-            const int32_t prev_head = atomicExch((int32_t*)&tab[slot] + 1, (int32_t)ga);  // little endian: high word = head
-            inc[ga] = prev_head == -2 ? -1 : prev_head;
+            allele_insert(arec, inc, tab, hmask, &univ[lo], &scal[1], ga, lo, ga - aoff[lo], d.anode + o, (int)(d.anode_off[a0 + ga + 1] - o), rankA[lo]);
         }
         __syncthreads();
         if (NEN > 0) {                                                  // the alignment nodes have landed
             while (true) { uint32_t ok; asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }" : "=r"(ok) : "r"(fr_smem_addr(&s_bar)), "r"(bar_phase) : "memory"); if (ok) break; }
             bar_phase ^= 1;
         }
-        // ---- S2: projection (k_project): one group of FR_G lanes per entry
+        // ---- S2: projection, one group of FR_G lanes per entry
         for (int e = grp; e < NE; e += NG) {
             const int rl = d.entry_read[e0 + e];
-            const float ident = d.entry_identity[e0 + e];
-            const bool good = good_identity(ident);
-            uint16_t* mrow = mask + rl * B;
-            const int32_t* nodes = enode_s + eoff[e];
-            const int Ln = eoff[e + 1] - eoff[e];
-            uint64_t ck = KEY_NONE, ckA = KEY_NONE;
-            for (int x0 = 0; x0 < Ln; x0 += FR_G) {
-                const int x = x0 + gl;
-                int32_t ga = -1, prev = 0, next = 0; bool has_prev = false, has_next = false;
-                if (x < Ln) {
-                    const int32_t v = nodes[x];
-                    has_prev = x > 0; has_next = x + 1 < Ln;
-                    if (has_prev) prev = nodes[x - 1];
-                    if (has_next) next = nodes[x + 1];
-                    uint32_t slot = hash_slot((uint32_t)v, hmask);
-                    while (true) {
-                        const unsigned long long sl = tab[slot];
-                        if (sl == SLOT_EMPTY) break;
-                        if ((uint32_t)sl == (uint32_t)v) { ga = (int32_t)(sl >> 32); break; }
-                        slot = (slot + 1) & hmask;
-                    }
-                }
-                while (__any_sync(gm, ga >= 0)) {
-                    const bool have = ga >= 0;
-                    int64_t o = 0; int len = 0;
-                    bool inner_ok = false, full_ok = false, slow = false;
-                    int4 rec = make_int4(0, 0, 0, 0);
-                    if (have) {
-                        rec = arec[ga];
-                        if (rec.x < 0) {                                                      // 3-node path
-                            inner_ok = true;
-                            full_ok = has_prev && has_next && ((prev == rec.y && next == rec.z) || (prev == rec.z && next == rec.y));
-                            slow = !full_ok;
-                        } else slow = true;
-                        if (slow) { o = d.anode_off[a0 + ga]; len = (int)(d.anode_off[a0 + ga + 1] - o); }
-                    }
-                    for (unsigned sm = __ballot_sync(gm, slow); sm; sm &= sm - 1) {
-                        const int src_lane = __ffs(sm) - 1;
-                        const int64_t oo = __shfl_sync(gm, o, src_lane);
-                        const int ll = __shfl_sync(gm, len, src_lane);
-                        bool in_ok = ll >= 3;
-                        for (int y = 2; in_ok && y < ll - 1; y++) in_ok = fr_entry_has(nodes, Ln, d.anode[oo + y], gl, gm);
-                        bool f_ok;
-                        if (ll >= 3) f_ok = in_ok && fr_entry_has(nodes, Ln, d.anode[oo], gl, gm) && fr_entry_has(nodes, Ln, d.anode[oo + ll - 1], gl, gm);
-                        else f_ok = (ll == 1) || fr_entry_has(nodes, Ln, d.anode[oo + 1], gl, gm);
-                        if (lane == src_lane) { inner_ok = in_ok; full_ok = f_ok; }
-                    }
-                    if (have) {
-                        const int b = (int)((uint32_t)rec.x & 0xfffffu);
-                        const int a = (int)(((uint32_t)rec.x >> 20) & 0xffu);
-                        const uint32_t bits = ((inner_ok && good) ? (1u << a) : 0u) | (full_ok ? 0x8000u : 0u);
-                        if (bits) atomic_or_u16(&mrow[b], (uint16_t)bits);
-                        if (inner_ok) { const uint64_t k = make_key((uint32_t)b, (uint32_t)a, (uint32_t)e); ck = k < ck ? k : ck; }
-                        if (full_ok) { const uint64_t k = make_key((uint32_t)rec.w, (uint32_t)a, (uint32_t)e); ckA = k < ckA ? k : ckA; }
-                        ga = inc[ga];
-                    }
-                }
-            }
-            ck = grp_min_u64<FR_G>(ck, gm); ckA = grp_min_u64<FR_G>(ckA, gm);
+            const bool good = good_identity(ident[e]);
+            uint64_t ck, ckA;
+            project_entry<FR_G, false>(enode_s + eoff[e], eoff[e + 1] - eoff[e], tab, hmask, arec, inc, d.anode_off + a0, d.anode, mask + rl * B,
+                                       good, (uint32_t)e, gm, ck, ckA);
             if (gl == 0) {
                 atomicMin(&fent[rl], (uint32_t)e); if (good) good_r[rl] = 1;
                 if (ck != KEY_NONE) atomicMin(&ckey[rl], (unsigned long long)ck);
@@ -223,97 +148,46 @@ __global__ void __launch_bounds__(FR_THREADS, 5) k_chain_front(DB d, int c_begin
             }
         }
         __syncthreads();
-        // ---- S3: stage-A statistics per read (k_read_stage_a)
+        // ---- S3: stage-A statistics per read
         for (int r = grp; r < R; r += NG) {
-            const uint16_t* mrow = mask + r * B;
-            int cnt = 0, first = INT32_MAX, last = -1;
-            for (int b = gl; b < B; b += FR_G) if (mrow[b] & 0x8000u) { cnt++; first = min(first, b); last = max(last, b); }
-            cnt = __reduce_add_sync(gm, cnt); first = __reduce_min_sync(gm, first); last = __reduce_max_sync(gm, last);
+            const int3 s = stage_a_row<FR_G>(mask + r * B, B, gl, gm);
             if (gl == 0) {
                 int mapq = 0;
-                if (cnt > 0) { mapq = mapq_of(d.entry_identity[e0 + (uint32_t)(ckeyA[r] & 0xffffffffu)]); atomicMax(&scal[0], last); }
-                rdA[r] = make_int4(cnt, first, last, mapq);
+                if (s.x > 0) { mapq = key_mapq(ident, ckeyA[r]); atomicMax(&scal[0], s.z); }
+                rdA[r] = make_int4(s.x, s.y, s.z, mapq);
             }
         }
         __syncthreads();
-        // ---- S4: boundary flags (k_chain_flags), to_be_added = [0, T) (k_chain_T)
-        {
-            const int mp = scal[0];
-            for (int r = tid; r < R; r += FR_THREADS) {
-                const int4 q = rdA[r];
-                if (!(q.x > 1 && q.w >= 93)) continue;
-                int f = 0;
-                if (q.z == mp) f |= 1;
-                if (q.z == mp - 1) f |= 2;
-                if (q.y == mp) f |= 4;
-                if (q.y == mp - 1) f |= 8;
-                if (f) atomicOr(&scal[1], f);
-            }
+        // ---- S4: boundary flags, to_be_added = [0, T)
+        for (int r = tid; r < R; r += FR_THREADS) {
+            const int4 q = rdA[r];
+            if (!read_passes(q.x, q.w)) continue;
+            const int f = boundary_flags(q.y, q.z, scal[0]);
+            if (f) atomicOr(&scal[1], f);
         }
         __syncthreads();
-        if (tid == 0) {
-            const int mp = scal[0], f = scal[1];
-            if (mp < 0) { scal[4] = AHS_CHAIN_EMPTY; scal[2] = 0; }                 // reference: UB (:193)
-            else {
-                const bool e_max = (f & 1) && !(f & 4), e_m1 = (f & 2) && !(f & 8);
-                int T = mp;
-                if (e_max) T = mp + 2; else if (e_m1) T = mp + 1;
-                scal[2] = min(T, B); scal[4] = AHS_CHAIN_OK;
-            }
-        }
+        if (tid == 0) scal[2] = chain_T(scal[0], scal[1], B, scal[4]);
         __syncthreads();
-        // ---- S5: final rows per read (k_read_rows)
+        // ---- S5: final rows per read
         {
             const int T = scal[2];
             const bool live = scal[4] == AHS_CHAIN_OK;
-            const bool has_univ = (scal[1] & CH_HAS_UNIV) != 0;
+            const uint32_t* univ_c = (scal[1] & CH_HAS_UNIV) ? univ : nullptr;
             for (int r = grp; r < R; r += NG) {
                 if (!live) { if (gl == 0) { rd[r] = make_int4(0, INT32_MAX, -1, 0); pass[r] = 0; } continue; }
-                uint16_t* mrow = mask + r * B;
-                const uint32_t fe = fent[r];
-                const bool has_entry = fe != 0xffffffffu;
-                const bool hg = good_r[r] != 0;
                 uint64_t ck = ckey[r];
-                if (has_entry && has_univ) for (int b = gl; b < T; b += FR_G) {
-                    const uint32_t u = univ[b];
-                    if (u != 0xffffffffu) { const uint64_t k = make_key((uint32_t)b, u, fe); ck = k < ck ? k : ck; }
-                }
-                ck = grp_min_u64<FR_G>(ck, gm);
-                const int bc = (ck == KEY_NONE) ? INT32_MAX : (int)(ck >> 40);
-                int nv = 0, last = -1;
-                if (bc < T) {
-                    const int ac = (int)((ck >> 32) & 0xff);
-                    for (int b = gl; b < B; b += FR_G) {
-                        uint32_t code = 0;
-                        if (b < T) {
-                            uint32_t m = mrow[b] & 0x7fffu;
-                            const uint32_t u = has_univ ? univ[b] : 0xffffffffu;
-                            if (u != 0xffffffffu && hg) m |= 1u << u;
-                            if (b == bc) code = (uint32_t)ac + 1u;
-                            else if (m) code = (uint32_t)__ffs((int)m);
-                        }
-                        mrow[b] = (uint16_t)code;
-                        if (code) { nv++; last = max(last, b); }
-                    }
-                    nv = __reduce_add_sync(gm, nv); last = __reduce_max_sync(gm, last);
-                } else for (int b = gl; b < B; b += FR_G) mrow[b] = 0;
-                int mapq = 0; bool ps = false;
-                if (bc < T) { mapq = mapq_of(d.entry_identity[e0 + (uint32_t)(ck & 0xffffffffu)]); ps = nv > 1 && mapq >= 93; }      // :270
-                __syncwarp(gm);
-                if (ps) for (int b = gl; b < T; b += FR_G) if (mrow[b]) poscov[b] = 1;
+                const RowOut o = final_row<FR_G>(mask + r * B, B, T, univ_c, fent[r], good_r[r] != 0, ck, ident, poscov, gl, gm);
                 if (gl == 0) {
-                    rd[r] = make_int4(nv, bc, last, mapq); pass[r] = ps ? 1 : 0; ckey[r] = ck;
-                    if (ps) { atomicAdd(&scal[3], 1); atomicAdd((unsigned long long*)&scal[6], (unsigned long long)nv); }
+                    rd[r] = make_int4(o.nv, o.first, o.last, o.mapq); pass[r] = o.pass ? 1 : 0; ckey[r] = ck;
+                    if (o.pass) { atomicAdd(&scal[3], 1); atomicAdd((unsigned long long*)&scal[6], (unsigned long long)o.nv); }
                 }
             }
         }
         __syncthreads();
-        // ---- S6: read order = order of the creation triples (k_read_rank), then ReadSet::sort() replayed (k_chain_sort); positions
+        // ---- S6: read order, then ReadSet::sort() replayed; positions
         for (int r = tid; r < R; r += FR_THREADS) {
             if (!pass[r]) continue;
-            const unsigned long long key = ckey[r];
-            int rank = 0;
-            for (int x = 0; x < R; x++) rank += (pass[x] && ckey[x] < key) ? 1 : 0;
+            const int rank = creation_rank(pass, (const uint64_t*)ckey, R, ckey[r]);
             ord[rank] = r; okey[rank] = rd[r].y;
         }
         __syncthreads();

@@ -17,6 +17,9 @@
 // hash table trigger node -> alleles turns the reference's bubbles x alleles x entries scan into
 // one lookup per entry node.  Paths without inner nodes match EVERY entry in stage B
 // (std::includes of an empty range, SURVEY A#9): they are kept per bubble as `bubble_univ`.
+//
+// Each rule is one __device__ function below, next to the kernel of this sequence that calls it; k_chain_front
+// (k_front.cuh) calls the same functions on its shared-memory copies of the chain's arrays.
 #pragma once
 #include "common.cuh"
 #include "device_batch.cuh"
@@ -49,38 +52,43 @@ __global__ void k_validate(DB d, int32_t* __restrict__ max_k) {
     if (bad) atomicOr(d.err_flags, bad);
 }
 
-// entry_read in range (needs entry_chain), stage_a_order values in range (needs bubble_chain)
+// an entry's read index names one of the R reads of its chain (err bit 8 otherwise)
+__device__ __forceinline__ bool entry_read_ok(int32_t r, int64_t R) { return r >= 0 && r < R; }
+
+// needs entry_chain
 __global__ void k_validate_owned(DB d) {
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x, x0 = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     int bad = 0;
-    for (int64_t e = x0; e < d.NE; e += stride) {
+    for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < d.NE; e += (int64_t)gridDim.x * blockDim.x) {
         const int c = d.entry_chain[e];
-        const int32_t r = d.entry_read[e];
-        if (r < 0 || r >= d.read_off[c + 1] - d.read_off[c]) bad |= 8;
-    }
-    if (d.stage_a_order) for (int64_t gb = x0; gb < d.NB; gb += stride) {
-        const int c = d.bubble_chain[gb];
-        const int32_t v = d.stage_a_order[gb];
-        if (v < 0 || v >= d.bubble_off[c + 1] - d.bubble_off[c]) bad |= 16;
+        if (!entry_read_ok(d.entry_read[e], d.read_off[c + 1] - d.read_off[c])) bad = 8;
     }
     if (bad) atomicOr(d.err_flags, bad);
 }
 
-// every slot of rankA written <=> stage_a_order is a permutation of each chain's bubble ids
-__global__ void k_validate_perm(DB d) {
-    for (int64_t gb = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; gb < d.NB; gb += (int64_t)gridDim.x * blockDim.x)
-        if (d.rankA[gb] < 0) atomicOr(d.err_flags, 16);
+// stage-A visit rank of bubble ob of a chain of B bubbles (inverse of stage_a_order, alignmentstoreadset.cpp:90; no order:
+// last bubble first).  false: the order's value is out of range (err bit 16).  Every slot of rankA written afterwards <=>
+// the order is a permutation of the chain's bubble ids.
+__device__ __forceinline__ bool rank_a_store(int32_t* rankA, const int32_t* order, int ob, int B) {
+    if (!order) { rankA[ob] = B - 1 - ob; return true; }
+    const int32_t v = order[ob];
+    if (v < 0 || v >= B) return false;
+    rankA[v] = ob;
+    return true;
 }
 
-// stage-A visit rank of each bubble (inverse of stage_a_order, alignmentstoreadset.cpp:90)
 __global__ void k_rank_a(DB d) {
     AHS_BAIL_ON_ERR(d);
     for (int64_t gb = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; gb < d.NB; gb += (int64_t)gridDim.x * blockDim.x) {
-        int c = d.bubble_chain[gb];
-        int64_t b0 = d.bubble_off[c];
-        if (d.stage_a_order) d.rankA[b0 + d.stage_a_order[gb]] = (int32_t)(gb - b0);
-        else d.rankA[gb] = (int32_t)(d.bubble_off[c + 1] - 1 - gb);
+        const int c = d.bubble_chain[gb];
+        const int64_t b0 = d.bubble_off[c];
+        if (!rank_a_store(d.rankA + b0, d.stage_a_order ? d.stage_a_order + b0 : nullptr, (int)(gb - b0), (int)(d.bubble_off[c + 1] - b0)))
+            atomicOr(d.err_flags, 16);
     }
+}
+
+__global__ void k_validate_perm(DB d) {
+    for (int64_t gb = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; gb < d.NB; gb += (int64_t)gridDim.x * blockDim.x)
+        if (d.rankA[gb] < 0) atomicOr(d.err_flags, 16);
 }
 
 // ---------------------------------------------------------------- K0: trigger table
@@ -88,6 +96,26 @@ __global__ void k_rank_a(DB d) {
 // chain), so that all probes of a chain's entries fall into a few KB that stay in L1/L2.  Slot = (head << 32 | node
 // id); all ones = empty; head = first allele of the list of alleles triggered by the node (inc_next links).
 constexpr unsigned long long SLOT_EMPTY = ~0ull;
+
+// allele a of bubble b (chain-local; ga its index into arec / inc): its 16-byte record for the projection (b | a << 20 |
+// 3-node flag << 31, end nodes, stage-A rank of b), its universal-allele minimum (*univ_b and the chain flag, A#9) and
+// its link into the list of its trigger node
+__device__ __forceinline__ void allele_insert(int4* arec, int32_t* inc, unsigned long long* tab, uint32_t hmask, uint32_t* univ_b,
+                                              int32_t* ch_flags, int32_t ga, int b, int a, const int32_t* path, int len, int32_t rank) {
+    arec[ga] = make_int4((int)((uint32_t)b | ((uint32_t)a << 20) | (len == 3 ? 0x80000000u : 0u)),
+                         len == 3 ? path[0] : 0, len == 3 ? path[2] : 0, rank);
+    if (len <= 2) { atomicMin(univ_b, (uint32_t)a); atomicOr(ch_flags, CH_HAS_UNIV); }
+    const uint32_t trig = (uint32_t)(len >= 3 ? path[1] : path[0]);
+    uint32_t slot = hash_slot(trig, hmask);
+    while (true) {
+        const unsigned long long claimed = (0xfffffffeull << 32) | trig;          // head = -2: no allele linked yet
+        const unsigned long long prev = atomicCAS(&tab[slot], SLOT_EMPTY, claimed);
+        if (prev == SLOT_EMPTY || (uint32_t)prev == trig) break;
+        slot = (slot + 1) & hmask;
+    }
+    const int32_t prev_head = atomicExch((int32_t*)&tab[slot] + 1, ga);            // little endian: high word = head
+    inc[ga] = prev_head == -2 ? -1 : prev_head;
+}
 
 __global__ void k_build_triggers(DB d) {
     AHS_BAIL_ON_ERR(d);
@@ -101,23 +129,8 @@ __global__ void k_build_triggers(DB d) {
         if (d.bubble_off[c + 1] - d.bubble_off[c] <= 1) continue;          // trivial chain: never phased (:86)
         const int a = (int)(ga - d.allele_off[gb]);
         if (a >= MAX_ALLELES) { atomicOr(d.err_flags, 2); continue; }
-        // everything k_project needs about a 3-node path in one 16-byte record: bubble (chain-local) | allele << 20 |
-        // simple-path flag << 31, end nodes, stage-A rank
-        d.arec[ga] = make_int4((int)((uint32_t)(gb - d.bubble_off[c]) | ((uint32_t)a << 20) | (len == 3 ? 0x80000000u : 0u)),
-                               len == 3 ? d.anode[o] : 0, len == 3 ? d.anode[o + 2] : 0, d.rankA[gb]);
-        if (len <= 2) { atomicMin(&d.bubble_univ[gb], (uint32_t)a); atomicOr(&d.ch_flags[c], CH_HAS_UNIV); }   // no inner node: matches every entry (A#9)
-        const uint32_t trig = (uint32_t)(len >= 3 ? d.anode[o + 1] : d.anode[o]);
-        unsigned long long* tab = d.hslots + d.hoff[c];
-        const uint32_t mask = d.hmaskc[c];
-        uint32_t slot = hash_slot(trig, mask);
-        while (true) {
-            const unsigned long long claimed = (0xfffffffeull << 32) | trig;          // head = -2: no allele linked yet
-            const unsigned long long prev = atomicCAS(&tab[slot], SLOT_EMPTY, claimed);
-            if (prev == SLOT_EMPTY || (uint32_t)prev == trig) break;
-            slot = (slot + 1) & mask;
-        }
-        const int32_t prev_head = atomicExch((int32_t*)&tab[slot] + 1, (int32_t)ga);  // little endian: high word = head
-        d.inc_next[ga] = prev_head == -2 ? -1 : prev_head;
+        allele_insert(d.arec, d.inc_next, d.hslots + d.hoff[c], d.hmaskc[c], &d.bubble_univ[gb], &d.ch_flags[c], (int32_t)ga,
+                      (int)(gb - d.bubble_off[c]), a, d.anode + o, len, d.rankA[gb]);
     }
 }
 
@@ -133,23 +146,95 @@ template <int G> __device__ __forceinline__ uint64_t grp_min_u64(uint64_t v, uns
 }
 
 // ---------------------------------------------------------------- K1: project entries
+// first allele triggered by node v (head of its list), -1 if none
+__device__ __forceinline__ int32_t trigger_lookup(const unsigned long long* tab, uint32_t hmask, int32_t v) {
+    uint32_t slot = hash_slot((uint32_t)v, hmask);
+    while (true) {
+        const unsigned long long sl = tab[slot];
+        if (sl == SLOT_EMPTY) return -1;
+        if ((uint32_t)sl == (uint32_t)v) return (int32_t)(sl >> 32);
+        slot = (slot + 1) & hmask;
+    }
+}
+
+// an entry's nodes in global memory (GMEM: through the read-only cache) or in shared memory, where __ldg must not go
+template <bool GMEM> __device__ __forceinline__ int32_t entry_node(const int32_t* p) {
+    if constexpr (GMEM) return __ldg(p); else return *p;
+}
+
 // is value q among the L nodes of the entry?  (whole lane group)
-template <int G>
-__device__ __forceinline__ bool grp_entry_has(const int32_t* __restrict__ nodes, int L, int32_t q, int gl, unsigned gm) {
+template <int G, bool GMEM>
+__device__ __forceinline__ bool entry_has(const int32_t* __restrict__ nodes, int L, int32_t q, int gl, unsigned gm) {
     bool f = false;
-    for (int x = gl; x < L; x += G) f |= __ldg(nodes + x) == q;
+    for (int x = gl; x < L; x += G) f |= entry_node<GMEM>(nodes + x) == q;
     return __any_sync(gm, f);
 }
 
-// one group of G lanes per alignment entry; lanes stride over the entry's nodes.  A node that is the trigger of an
-// allele path (hash hit) decides the two containment tests of the reference (is_subset with and without the end
-// nodes, :495-548).  Common case, decided by the lane alone: a 3-node path whose end nodes are the neighbours of
-// the trigger in the alignment.  Everything else is decided by the whole group scanning the entry.
+// One group of G lanes projects one alignment entry (index el within its chain) onto its read's mask row; lanes stride over
+// the entry's nodes.  A node that is the trigger of an allele path (hash hit) decides the two containment tests of the
+// reference (is_subset with and without the end nodes, :495-548).  Common case, decided by the lane alone: a 3-node path
+// whose end nodes are the neighbours of the trigger in the alignment.  Everything else is decided by the whole group
+// scanning the entry.  arec, inc and anode_off are indexed by the allele ids the table holds.  Returns, on every lane of
+// the group, the smallest creation keys (position | allele | entry) of the stage-B (ck) and stage-A (ckA) matches.
+template <int G, bool GMEM>
+__device__ __forceinline__ void project_entry(const int32_t* __restrict__ nodes, int L, const unsigned long long* tab, uint32_t hmask,
+                                              const int4* arec, const int32_t* inc, const int64_t* anode_off, const int32_t* anode,
+                                              uint16_t* mrow, bool good, uint32_t el, unsigned gm, uint64_t& ck_out, uint64_t& ckA_out) {
+    const int lane = lane_id(), gl = lane % G;
+    uint64_t ck = KEY_NONE, ckA = KEY_NONE;                 // smallest creation keys seen by this lane
+    for (int x0 = 0; x0 < L; x0 += G) {
+        const int x = x0 + gl;
+        int32_t ga = -1, prev = 0, next = 0; bool has_prev = false, has_next = false;
+        if (x < L) {
+            has_prev = x > 0; has_next = x + 1 < L;
+            if (has_prev) prev = entry_node<GMEM>(nodes + x - 1);
+            if (has_next) next = entry_node<GMEM>(nodes + x + 1);
+            ga = trigger_lookup(tab, hmask, entry_node<GMEM>(nodes + x));
+        }
+        while (__any_sync(gm, ga >= 0)) {
+            const bool have = ga >= 0;
+            int64_t o = 0; int len = 0;
+            bool inner_ok = false, full_ok = false, slow = false;
+            int4 rec = make_int4(0, 0, 0, 0);
+            if (have) {
+                rec = arec[ga];
+                if (rec.x < 0) {                                                      // 3-node path
+                    inner_ok = true;                                                  // the only inner node is the trigger
+                    full_ok = has_prev && has_next && ((prev == rec.y && next == rec.z) || (prev == rec.z && next == rec.y));
+                    slow = !full_ok;                                                  // the end nodes may still be elsewhere in the entry
+                } else slow = true;
+                if (slow) { o = anode_off[ga]; len = (int)(anode_off[ga + 1] - o); }
+            }
+            for (unsigned sm = __ballot_sync(gm, slow); sm; sm &= sm - 1) {
+                const int src_lane = __ffs(sm) - 1;                                   // absolute lane, inside this group
+                const int64_t oo = __shfl_sync(gm, o, src_lane);
+                const int ll = __shfl_sync(gm, len, src_lane);
+                bool in_ok = ll >= 3;                          // len <= 2: universal, handled by final_row
+                for (int y = 2; in_ok && y < ll - 1; y++) in_ok = entry_has<G, GMEM>(nodes, L, anode[oo + y], gl, gm);
+                bool f_ok;
+                if (ll >= 3) f_ok = in_ok && entry_has<G, GMEM>(nodes, L, anode[oo], gl, gm) && entry_has<G, GMEM>(nodes, L, anode[oo + ll - 1], gl, gm);
+                else f_ok = (ll == 1) || entry_has<G, GMEM>(nodes, L, anode[oo + 1], gl, gm);
+                if (lane == src_lane) { inner_ok = in_ok; full_ok = f_ok; }
+            }
+            if (have) {
+                const int b = (int)((uint32_t)rec.x & 0xfffffu);
+                const int a = (int)(((uint32_t)rec.x >> 20) & 0xffu);
+                const uint32_t bits = ((inner_ok && good) ? (1u << a) : 0u) | (full_ok ? 0x8000u : 0u);
+                if (bits) atomic_or_u16(&mrow[b], (uint16_t)bits);                   // one atomic for both tests
+                if (inner_ok) { const uint64_t k = make_key((uint32_t)b, (uint32_t)a, el); ck = k < ck ? k : ck; }
+                if (full_ok) { const uint64_t k = make_key((uint32_t)rec.w, (uint32_t)a, el); ckA = k < ckA ? k : ckA; }
+                ga = inc[ga];
+            }
+        }
+    }
+    ck_out = grp_min_u64<G>(ck, gm); ckA_out = grp_min_u64<G>(ckA, gm);
+}
+
 template <int G>
 __global__ void __launch_bounds__(256, 6) k_project(DB d, int64_t e_begin, int64_t e_end) {
     AHS_BAIL_ON_ERR(d);
     const unsigned gm = grp_mask<G>();
-    const int lane = lane_id(), gl = lane % G;
+    const int gl = lane_id() % G;
     const int64_t gpb = blockDim.x / G, g0 = blockIdx.x * gpb + threadIdx.x / G;
     for (int64_t ge = e_begin + g0; ge < e_end; ge += (int64_t)gridDim.x * gpb) {
         const int c = d.entry_chain[ge];
@@ -159,67 +244,10 @@ __global__ void __launch_bounds__(256, 6) k_project(DB d, int64_t e_begin, int64
         const int rl = d.entry_read[ge];
         const int64_t r = d.read_off[c] + rl;
         const uint32_t el = (uint32_t)(ge - d.entry_off[c]);
-        const float ident = d.entry_identity[ge];
-        const bool good = good_identity(ident);
-        uint16_t* mrow = d.mask + d.mrow_off[c] + (int64_t)rl * B;
-        const int32_t* nodes = d.enode + d.enode_off[ge];
-        const int L = (int)(d.enode_off[ge + 1] - d.enode_off[ge]);
-        const unsigned long long* tab = d.hslots + d.hoff[c];
-        const uint32_t mask = d.hmaskc[c];
-        uint64_t ck = KEY_NONE, ckA = KEY_NONE;                 // smallest creation keys seen by this lane
-        for (int x0 = 0; x0 < L; x0 += G) {
-            const int x = x0 + gl;
-            int32_t ga = -1, prev = 0, next = 0; bool has_prev = false, has_next = false;
-            if (x < L) {
-                const int32_t v = __ldg(nodes + x);
-                has_prev = x > 0; has_next = x + 1 < L;
-                if (has_prev) prev = __ldg(nodes + x - 1);
-                if (has_next) next = __ldg(nodes + x + 1);
-                uint32_t slot = hash_slot((uint32_t)v, mask);
-                while (true) {
-                    const unsigned long long sl = tab[slot];
-                    if (sl == SLOT_EMPTY) break;
-                    if ((uint32_t)sl == (uint32_t)v) { ga = (int32_t)(sl >> 32); break; }
-                    slot = (slot + 1) & mask;
-                }
-            }
-            while (__any_sync(gm, ga >= 0)) {
-                const bool have = ga >= 0;
-                int64_t gb = 0, o = 0; int len = 0;
-                bool inner_ok = false, full_ok = false, slow = false;
-                int4 rec = make_int4(0, 0, 0, 0);
-                if (have) {
-                    rec = d.arec[ga];
-                    if (rec.x < 0) {                                                      // 3-node path
-                        inner_ok = true;                                                  // the only inner node is the trigger
-                        full_ok = has_prev && has_next && ((prev == rec.y && next == rec.z) || (prev == rec.z && next == rec.y));
-                        slow = !full_ok;                                                  // the end nodes may still be elsewhere in the entry
-                    } else slow = true;
-                    if (slow) { gb = d.allele_bubble[ga]; o = d.anode_off[ga]; len = (int)(d.anode_off[ga + 1] - o); }
-                }
-                for (unsigned sm = __ballot_sync(gm, slow); sm; sm &= sm - 1) {
-                    const int src_lane = __ffs(sm) - 1;                                   // absolute lane, inside this group
-                    const int64_t oo = __shfl_sync(gm, o, src_lane);
-                    const int ll = __shfl_sync(gm, len, src_lane);
-                    bool in_ok = ll >= 3;                          // len <= 2: universal, handled in k_read_rows
-                    for (int y = 2; in_ok && y < ll - 1; y++) in_ok = grp_entry_has<G>(nodes, L, d.anode[oo + y], gl, gm);
-                    bool f_ok;
-                    if (ll >= 3) f_ok = in_ok && grp_entry_has<G>(nodes, L, d.anode[oo], gl, gm) && grp_entry_has<G>(nodes, L, d.anode[oo + ll - 1], gl, gm);
-                    else f_ok = (ll == 1) || grp_entry_has<G>(nodes, L, d.anode[oo + 1], gl, gm);
-                    if (lane == src_lane) { inner_ok = in_ok; full_ok = f_ok; }
-                }
-                if (have) {
-                    const int b = (int)((uint32_t)rec.x & 0xfffffu);
-                    const int a = (int)(((uint32_t)rec.x >> 20) & 0xffu);
-                    const uint32_t bits = ((inner_ok && good) ? (1u << a) : 0u) | (full_ok ? 0x8000u : 0u);
-                    if (bits) atomic_or_u16(&mrow[b], (uint16_t)bits);                   // one atomic for both tests
-                    if (inner_ok) { const uint64_t k = make_key((uint32_t)b, (uint32_t)a, el); ck = k < ck ? k : ck; }
-                    if (full_ok) { const uint64_t k = make_key((uint32_t)rec.w, (uint32_t)a, el); ckA = k < ckA ? k : ckA; }
-                    ga = d.inc_next[ga];
-                }
-            }
-        }
-        ck = grp_min_u64<G>(ck, gm); ckA = grp_min_u64<G>(ckA, gm);
+        const bool good = good_identity(d.entry_identity[ge]);
+        uint64_t ck, ckA;
+        project_entry<G, true>(d.enode + d.enode_off[ge], (int)(d.enode_off[ge + 1] - d.enode_off[ge]), d.hslots + d.hoff[c], d.hmaskc[c],
+                               d.arec, d.inc_next, d.anode_off, d.anode, d.mask + d.mrow_off[c] + (int64_t)rl * B, good, el, gm, ck, ckA);
         if (gl == 0) {
             atomicMin(&d.first_entry[r], el); if (good) d.has_good[r] = 1;
             if (ck != KEY_NONE) atomicMin((unsigned long long*)&d.create_key[r], (unsigned long long)ck);
@@ -229,7 +257,20 @@ __global__ void __launch_bounds__(256, 6) k_project(DB d, int64_t e_begin, int64
 }
 
 // ---------------------------------------------------------------- K1b: stage-A statistics per read
-// count / first / last fully contained bubble and the stage-A mapq (:146-165, :173-182)
+// count / first / last fully contained bubble of a read's mask row (:146-165), reduced over the group
+template <int G>
+__device__ __forceinline__ int3 stage_a_row(const uint16_t* mrow, int B, int gl, unsigned gm) {
+    int cnt = 0, first = INT32_MAX, last = -1;
+    for (int b = gl; b < B; b += G) if (mrow[b] & 0x8000u) { cnt++; first = min(first, b); last = max(last, b); }
+    return make_int3(__reduce_add_sync(gm, cnt), __reduce_min_sync(gm, first), __reduce_max_sync(gm, last));
+}
+
+// mapq of a read: that of the entry in its creation key (ident: the identities of the chain's entries; :117, :234)
+__device__ __forceinline__ int32_t key_mapq(const float* ident, uint64_t key) { return mapq_of(ident[(uint32_t)(key & 0xffffffffu)]); }
+
+// the read filter of stage A and of the final read set (:173-182, :270)
+__device__ __forceinline__ bool read_passes(int n, int32_t mapq) { return n > 1 && mapq >= 93; }
+
 template <int G>
 __global__ void __launch_bounds__(256) k_read_stage_a(DB d) {
     AHS_BAIL_ON_ERR(d);
@@ -240,58 +281,103 @@ __global__ void __launch_bounds__(256) k_read_stage_a(DB d) {
         const int c = d.read_chain[r];
         const int B = (int)(d.bubble_off[c + 1] - d.bubble_off[c]);
         if (B <= 1) continue;
-        const uint16_t* mrow = d.mask + d.mrow_off[c] + (r - d.read_off[c]) * B;
-        int cnt = 0, first = INT32_MAX, last = -1;
-        for (int b = gl; b < B; b += G) if (mrow[b] & 0x8000u) { cnt++; first = min(first, b); last = max(last, b); }
-        cnt = __reduce_add_sync(gm, cnt); first = __reduce_min_sync(gm, first); last = __reduce_max_sync(gm, last);
+        const int3 s = stage_a_row<G>(d.mask + d.mrow_off[c] + (r - d.read_off[c]) * B, B, gl, gm);
         if (gl == 0) {
             int mapq = 0;
-            if (cnt > 0) {
-                const uint32_t el = (uint32_t)(d.createA_key[r] & 0xffffffffu);
-                mapq = mapq_of(d.entry_identity[d.entry_off[c] + el]);
-                atomicMax(&d.ch_maxpos[c], last);
-            }
-            d.rdA_cnt[r] = cnt; d.rdA_first[r] = first; d.rdA_last[r] = last; d.rdA_mapq[r] = mapq;
+            if (s.x > 0) { mapq = key_mapq(d.entry_identity + d.entry_off[c], d.createA_key[r]); atomicMax(&d.ch_maxpos[c], s.z); }
+            d.rdA_cnt[r] = s.x; d.rdA_first[r] = s.y; d.rdA_last[r] = s.z; d.rdA_mapq[r] = mapq;
         }
     }
 }
 
-// boundary flags: which of maxpos-1 / maxpos are last / first positions of filtered stage-A reads (:173-189)
+// boundary flags of a filtered stage-A read: which of maxpos-1 / maxpos are its last (1, 2) or first (4, 8) position (:173-189)
+__device__ __forceinline__ int boundary_flags(int first, int last, int mp) {
+    int f = 0;
+    if (last == mp) f |= 1;
+    if (last == mp - 1) f |= 2;
+    if (first == mp) f |= 4;
+    if (first == mp - 1) f |= 8;
+    return f;
+}
+
 __global__ void k_chain_flags(DB d) {
     AHS_BAIL_ON_ERR(d);
     for (int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; r < d.NR; r += (int64_t)gridDim.x * blockDim.x) {
         const int c = d.read_chain[r];
         if (d.bubble_off[c + 1] - d.bubble_off[c] <= 1) continue;
-        if (!(d.rdA_cnt[r] > 1 && d.rdA_mapq[r] >= 93)) continue;
-        const int mp = d.ch_maxpos[c];
-        int f = 0;
-        if (d.rdA_last[r] == mp) f |= 1;
-        if (d.rdA_last[r] == mp - 1) f |= 2;
-        if (d.rdA_first[r] == mp) f |= 4;
-        if (d.rdA_first[r] == mp - 1) f |= 8;
+        if (!read_passes(d.rdA_cnt[r], d.rdA_mapq[r])) continue;
+        const int f = boundary_flags(d.rdA_first[r], d.rdA_last[r], d.ch_maxpos[c]);
         if (f) atomicOr(&d.ch_flags[c], f);
     }
 }
 
-// to_be_added = [0,maxpos) U {e, e+1 : e in last \ first} = [0, T)  (:173-209, SURVEY A#10)
+// to_be_added = [0,maxpos) U {e, e+1 : e in last \ first} = [0, T) of a chain of B > 1 bubbles, from maxpos mp and the
+// boundary flags f; `status` = OK, or EMPTY when no read contains a full bubble path (:173-209, SURVEY A#10)
+__device__ __forceinline__ int chain_T(int mp, int f, int B, int32_t& status) {
+    if (mp < 0) { status = AHS_CHAIN_EMPTY; return 0; }          // reference: UB (:193)
+    const bool e_max = (f & 1) && !(f & 4);          // maxpos   in last \ first  -> adds maxpos, maxpos+1
+    const bool e_m1  = (f & 2) && !(f & 8);          // maxpos-1 in last \ first  -> adds maxpos-1, maxpos
+    int T = mp;
+    if (e_max) T = mp + 2; else if (e_m1) T = mp + 1;
+    status = AHS_CHAIN_OK;
+    return min(T, B);                                  // bubble ids >= B have no alleles (:216 default-insert)
+}
+
 __global__ void k_chain_T(DB d) {
     AHS_BAIL_ON_ERR(d);
     for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < d.C; c += gridDim.x * blockDim.x) {
         const int B = (int)(d.bubble_off[c + 1] - d.bubble_off[c]);
         if (B <= 1) { d.ch_status[c] = AHS_CHAIN_TRIVIAL; d.ch_T[c] = 0; continue; }
-        const int mp = d.ch_maxpos[c];
-        if (mp < 0) { d.ch_status[c] = AHS_CHAIN_EMPTY; d.ch_T[c] = 0; continue; }   // reference: UB (:193)
-        const int f = d.ch_flags[c];
-        const bool e_max = (f & 1) && !(f & 4);          // maxpos   in last \ first  -> adds maxpos, maxpos+1
-        const bool e_m1  = (f & 2) && !(f & 8);          // maxpos-1 in last \ first  -> adds maxpos-1, maxpos
-        int T = mp;
-        if (e_max) T = mp + 2; else if (e_m1) T = mp + 1;
-        d.ch_T[c] = min(T, B);                             // bubble ids >= B have no alleles (:216 default-insert)
-        d.ch_status[c] = AHS_CHAIN_OK;
+        int32_t status;
+        d.ch_T[c] = chain_T(d.ch_maxpos[c], d.ch_flags[c], B, status);
+        d.ch_status[c] = status;
     }
 }
 
 // ---------------------------------------------------------------- K1d: final rows per read (stage B + filter)
+struct RowOut { int nv, first, last, mapq; bool pass; };
+
+// Stage B and the filter for one read, to_be_added = [0, T) (:210-254, :262-270), by the whole group.  ck: the read's
+// creation key, updated with the universal alleles (univ: nullptr if the chain has none; fe: the read's first entry).
+// A read created below T gets its row rewritten into allele codes and, if it passes, its positions marked in poscov;
+// other rows stay as projected, because only the rows of final reads are read afterwards.
+template <int G>
+__device__ __forceinline__ RowOut final_row(uint16_t* mrow, int B, int T, const uint32_t* univ, uint32_t fe, bool hg, uint64_t& ck,
+                                            const float* ident, uint8_t* poscov, int gl, unsigned gm) {
+    if (fe != 0xffffffffu && univ) for (int b = gl; b < T; b += G) {
+        const uint32_t u = univ[b];
+        if (u != 0xffffffffu) { const uint64_t k = make_key((uint32_t)b, u, fe); ck = k < ck ? k : ck; }
+    }
+    ck = grp_min_u64<G>(ck, gm);
+    RowOut o; o.nv = 0; o.first = (ck == KEY_NONE) ? INT32_MAX : (int)(ck >> 40); o.last = -1; o.mapq = 0; o.pass = false;
+    uint32_t cov = 0;                                                   // this lane's covered positions b = gl + G j, j < 32
+    if (o.first < T) {
+        const int ac = (int)((ck >> 32) & 0xff);
+        int nv = 0, last = -1;
+        for (int b = gl; b < B; b += G) {
+            uint32_t code = 0;
+            if (b < T) {
+                uint32_t m = mrow[b] & 0x7fffu;
+                const uint32_t u = univ ? univ[b] : 0xffffffffu;
+                if (u != 0xffffffffu && hg) m |= 1u << u;
+                if (b == o.first) code = (uint32_t)ac + 1u;
+                else if (m) code = (uint32_t)__ffs((int)m);             // lowest set bit = first matching allele
+            }
+            mrow[b] = (uint16_t)code;
+            if (code) { nv++; last = max(last, b); if (b < 32 * G) cov |= 1u << (b / G); }
+        }
+        o.nv = __reduce_add_sync(gm, nv); o.last = __reduce_max_sync(gm, last);
+        o.mapq = key_mapq(ident, ck);
+        o.pass = read_passes(o.nv, o.mapq);
+    }
+    __syncwarp(gm);                                                     // the group's codes are written
+    if (o.pass) {
+        for (uint32_t m = cov; m; m &= m - 1) poscov[gl + G * (__ffs((int)m) - 1)] = 1;   // codes are only set below T
+        for (int b = gl + 32 * G; b < T; b += G) if (mrow[b]) poscov[b] = 1;
+    }
+    return o;
+}
+
 template <int G>
 __global__ void __launch_bounds__(256) k_read_rows(DB d) {
     AHS_BAIL_ON_ERR(d);
@@ -305,52 +391,14 @@ __global__ void __launch_bounds__(256) k_read_rows(DB d) {
         if (d.ch_status[c] != AHS_CHAIN_OK) continue;
         const int64_t b0g = d.bubble_off[c];
         const int B = (int)(d.bubble_off[c + 1] - b0g);
-        const int T = d.ch_T[c];
-        uint16_t* mrow = d.mask + d.mrow_off[c] + (r - d.read_off[c]) * B;
-        const uint32_t fe = d.first_entry[r];
-        const bool has_entry = fe != 0xffffffffu;
-        const bool hg = d.has_good[r] != 0;
         const bool univ = (d.ch_flags[c] & CH_HAS_UNIV) != 0;              // rare: a bubble with an allele path of <= 2 nodes
-        // creation triple: minimum (position, allele, entry) over all matches, universal alleles included
         uint64_t ck = d.create_key[r];
-        if (has_entry && univ) for (int b = gl; b < T; b += G) {
-            const uint32_t u = d.bubble_univ[b0g + b];
-            if (u != 0xffffffffu) { uint64_t k = make_key((uint32_t)b, u, fe); ck = k < ck ? k : ck; }
-        }
-        ck = grp_min_u64<G>(ck, gm);
-        const int bc = (ck == KEY_NONE) ? INT32_MAX : (int)(ck >> 40);
-        int nv = 0, last = -1;
-        uint32_t cov = 0;                                                   // this lane's covered positions b = gl + G j, j < 32
-        if (bc < T) {
-            const int ac = (int)((ck >> 32) & 0xff);
-            for (int b = gl; b < B; b += G) {
-                uint32_t code = 0;
-                if (b < T) {
-                    uint32_t m = mrow[b] & 0x7fffu;
-                    const uint32_t u = univ ? d.bubble_univ[b0g + b] : 0xffffffffu;
-                    if (u != 0xffffffffu && hg) m |= 1u << u;
-                    if (b == bc) code = (uint32_t)ac + 1u;
-                    else if (m) code = (uint32_t)__ffs((int)m);             // lowest set bit = first matching allele
-                }
-                mrow[b] = (uint16_t)code;
-                if (code) { nv++; last = max(last, b); if (b < 32 * G) cov |= 1u << (b / G); }
-            }
-            nv = __reduce_add_sync(gm, nv); last = __reduce_max_sync(gm, last);
-        }
-        int mapq = 0; bool pass = false;
-        if (bc < T) {
-            mapq = mapq_of(d.entry_identity[d.entry_off[c] + (uint32_t)(ck & 0xffffffffu)]);
-            pass = nv > 1 && mapq >= 93;                                    // :270
-        }
-        __syncwarp(gm);                                                     // the group's codes are written
-        if (pass) {
-            for (uint32_t m = cov; m; m &= m - 1) d.poscov[b0g + gl + G * (__ffs((int)m) - 1)] = 1;   // codes are only set below T
-            for (int b = gl + 32 * G; b < T; b += G) if (mrow[b]) d.poscov[b0g + b] = 1;
-        }
+        const RowOut o = final_row<G>(d.mask + d.mrow_off[c] + (r - d.read_off[c]) * B, B, d.ch_T[c], univ ? d.bubble_univ + b0g : nullptr,
+                                      d.first_entry[r], d.has_good[r] != 0, ck, d.entry_identity + d.entry_off[c], d.poscov + b0g, gl, gm);
         if (gl == 0) {
-            d.rd_nv[r] = nv; d.rd_first[r] = bc; d.rd_last[r] = last; d.rd_mapq[r] = mapq; d.rd_pass[r] = pass ? 1 : 0;
+            d.rd_nv[r] = o.nv; d.rd_first[r] = o.first; d.rd_last[r] = o.last; d.rd_mapq[r] = o.mapq; d.rd_pass[r] = o.pass ? 1 : 0;
             d.create_key[r] = ck;
-            if (pass) { atomicAdd(&d.ch_nfinal[c], 1); atomicAdd(&d.ch_cells[c], (unsigned long long)nv); cells_local += nv; }
+            if (o.pass) { atomicAdd(&d.ch_nfinal[c], 1); atomicAdd(&d.ch_cells[c], (unsigned long long)o.nv); cells_local += o.nv; }
         }
     }
     // one atomic per warp on the batch-wide cell counter (a per-read atomic on one address serialises in L2)
@@ -360,16 +408,21 @@ __global__ void __launch_bounds__(256) k_read_rows(DB d) {
 }
 
 // ---------------------------------------------------------------- K1e: read order
-// Insertion order of the stage-B read set = order of the creation triples; rank by counting.
+// Insertion order of the stage-B read set = order of the creation triples: the rank of a passing read's key among the n
+// reads of its chain, by counting.
+__device__ __forceinline__ int creation_rank(const uint8_t* pass, const uint64_t* key, int n, uint64_t k) {
+    int rank = 0;
+    for (int x = 0; x < n; x++) rank += (pass[x] && key[x] < k) ? 1 : 0;
+    return rank;
+}
+
 __global__ void k_read_rank(DB d) {
     AHS_BAIL_ON_ERR(d);
     for (int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; r < d.NR; r += (int64_t)gridDim.x * blockDim.x) {
         if (!d.rd_pass[r]) continue;
         const int c = d.read_chain[r];
-        const int64_t r0 = d.read_off[c], r1 = d.read_off[c + 1];
-        const uint64_t key = d.create_key[r];
-        int rank = 0;
-        for (int64_t x = r0; x < r1; x++) rank += (d.rd_pass[x] && d.create_key[x] < key) ? 1 : 0;
+        const int64_t r0 = d.read_off[c];
+        const int rank = creation_rank(d.rd_pass + r0, d.create_key + r0, (int)(d.read_off[c + 1] - r0), d.create_key[r]);
         d.ord[r0 + rank] = (int32_t)(r - r0);
         d.okey[r0 + rank] = d.rd_first[r];
     }

@@ -468,7 +468,7 @@ struct Pipeline {
             if (sz.NA) k_owner<<<grid_for(sz.NA, TB, sms), TB, 0, st>>>(d.allele_off, (int)sz.NB, sz.NA, d.allele_bubble); n_launches += 1;
             if (sz.NE) k_owner<<<grid_for(sz.NE, TB, sms), TB, 0, st>>>(d.entry_off, (int)C, sz.NE, d.entry_chain); n_launches += 1;
             if (sz.NR) k_owner<<<grid_for(sz.NR, TB, sms), TB, 0, st>>>(d.read_off, (int)C, sz.NR, d.read_chain); n_launches += 1;
-            k_validate_owned<<<grid_for(std::max(sz.NE, sz.NB), TB, sms), TB, 0, st>>>(d); n_launches += 1;
+            k_validate_owned<<<grid_for(sz.NE, TB, sms), TB, 0, st>>>(d); n_launches += 1;
             if (sz.NB) k_rank_a<<<grid_for(sz.NB, TB, sms), TB, 0, st>>>(d); n_launches += 1;
             if (sz.NB && d.stage_a_order) { k_validate_perm<<<grid_for(sz.NB, TB, sms), TB, 0, st>>>(d); n_launches += 1; }
             if (sz.NA) k_build_triggers<<<grid_for(sz.NA, TB, sms), TB, 0, st>>>(d); n_launches += 1;

@@ -307,19 +307,27 @@ def test_chunked_call_is_result_identical(chunks, monkeypatch):
     assert not api.phase_batch(b).diff(want)
 
 
+_DEL_ANODE = [1, 2, 4, 1, 3, 4,   4, 5, 7, 7, 4,   7, 8, 10, 7, 9, 10]
+_DEL_ANODE_OFF = [0, 3, 6, 9, 11, 14, 17]
+_DEL_ALLELE_OFF = [0, 2, 4, 6]
+_DEL_READS = [[1, 2, 4, 5, 7, 8, 10], [1, 3, 4, 7, 9, 10], [1, 2, 4], [7, 8, 10, 4, 5], [1, 3, 4, 5, 7, 9, 10]]
+
+
+def deletion_allele_chain():
+    """One diploid chain of three bubbles whose middle bubble has the allele path 7-4: two nodes, no inner node."""
+    n = len(_DEL_READS)
+    return api.Batch(2, [0], [0, 3], _DEL_ALLELE_OFF, _DEL_ANODE_OFF, _DEL_ANODE, [2, 1, 0], [0, n], [0, n],
+                     np.cumsum([0] + [len(x) for x in _DEL_READS]), sum(_DEL_READS, []), list(range(n)), [0.99] * n)
+
+
 def test_deletion_allele_matches_every_entry():
     # allele path of two nodes (no inner node): stage B matches it for every entry of the chain (SURVEY A#9); same hand-made
     # chain as tests/test_oracle_cpu.py, alone and next to ordinary chains (the per-chain "has universal allele" flag)
     from ahsoka_b200.api import Batch
-    anode = [1, 2, 4, 1, 3, 4,   4, 5, 7, 7, 4,   7, 8, 10, 7, 9, 10]
-    anode_off = [0, 3, 6, 9, 11, 14, 17]
-    allele_off = [0, 2, 4, 6]
-    reads = [[1, 2, 4, 5, 7, 8, 10], [1, 3, 4, 7, 9, 10], [1, 2, 4], [7, 8, 10, 4, 5], [1, 3, 4, 5, 7, 9, 10]]
+    anode, anode_off, allele_off, reads = _DEL_ANODE, _DEL_ANODE_OFF, _DEL_ALLELE_OFF, _DEL_READS
     enode = sum(reads, [])
     enode_off = np.cumsum([0] + [len(x) for x in reads])
-    b = Batch(2, [0], [0, 3], allele_off, anode_off, anode, [2, 1, 0], [0, len(reads)], [0, len(reads)], enode_off, enode,
-              list(range(len(reads))), [0.99] * len(reads))
-    got = _check(b)
+    got = _check(deletion_allele_chain())
     assert got.status[0] == 0
     # the same chain between two synthetic ones
     s = synth.generate(synth.params(2, 2, 1, 12, depth=20.0, seed=333))
