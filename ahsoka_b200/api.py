@@ -64,6 +64,9 @@ class Batch:
     entry_read: np.ndarray
     entry_identity: np.ndarray
     truth: dict = field(default_factory=dict)
+    # optional caller genotypes, one uint8 per allele (indexed like allele_off): how many haplotypes carry the allele.
+    # Per bubble all 0 (unknown) or summing to the ploidy; see ahs_phase_batch_genotyped in include/ahsoka_b200.h.
+    allele_dosage: np.ndarray | None = None
 
     def __post_init__(self):
         for k in _I32:
@@ -71,6 +74,15 @@ class Batch:
         for k in _I64:
             setattr(self, k, np.ascontiguousarray(getattr(self, k), dtype=np.int64))
         self.entry_identity = np.ascontiguousarray(self.entry_identity, dtype=np.float32)
+        if self.allele_dosage is not None:
+            self.allele_dosage = np.ascontiguousarray(self.allele_dosage, dtype=np.uint8)
+
+    def dosage_ptr(self):
+        """ctypes pointer to allele_dosage, after checking that it has one entry per allele."""
+        n_alleles = int(self.allele_off[-1]) if len(self.allele_off) else 0
+        if self.allele_dosage.shape != (n_alleles,):
+            raise ValueError(f"allele_dosage has shape {self.allele_dosage.shape}, the batch has {n_alleles} alleles")
+        return self.allele_dosage.ctypes.data_as(u8p)
 
     @property
     def n_chains(self):
@@ -115,18 +127,21 @@ class Batch:
         np.cumsum(r_n, out=r_off[1:])
         return Batch(self.ploidy, self.chain_id[chains], b_off, a_off_rel, an_off, self.anode[an_idx],
                      self.stage_a_order[b_idx], r_off, e_off, en_off, self.enode[en_idx],
-                     self.entry_read[e_idx], self.entry_identity[e_idx])
+                     self.entry_read[e_idx], self.entry_identity[e_idx],
+                     allele_dosage=None if self.allele_dosage is None else self.allele_dosage[a_idx])
 
     def save(self, path):
+        extra = {} if self.allele_dosage is None else {"allele_dosage": self.allele_dosage}
         np.savez_compressed(path, ploidy=self.ploidy, **{k: getattr(self, k) for k in _I32 + _I64},
-                            entry_identity=self.entry_identity)
+                            entry_identity=self.entry_identity, **extra)
 
     @staticmethod
     def load(path) -> "Batch":
         z = np.load(path)
         return Batch(int(z["ploidy"]), *[z[k] for k in ("chain_id", "bubble_off", "allele_off", "anode_off", "anode",
                                                         "stage_a_order", "read_off", "entry_off", "enode_off", "enode",
-                                                        "entry_read", "entry_identity")])
+                                                        "entry_read", "entry_identity")],
+                     allele_dosage=z["allele_dosage"] if "allele_dosage" in z.files else None)
 
     @staticmethod
     def from_dump(path) -> "Batch":
@@ -250,6 +265,8 @@ def load_library(path: str = LIB_PATH):
     lib.ahs_phase_batch_multi.restype = C.c_int
     lib.ahs_phase_batch_resident.argtypes = [C.POINTER(BatchIn), C.POINTER(BatchOut), C.c_int, C.c_int, C.c_int]
     lib.ahs_phase_batch_resident.restype = C.c_int
+    lib.ahs_phase_batch_genotyped.argtypes = [C.POINTER(BatchIn), u8p, C.POINTER(BatchOut), C.POINTER(C.c_int), C.c_int]
+    lib.ahs_phase_batch_genotyped.restype = C.c_int
     lib.ahs_free_out.argtypes = [C.POINTER(BatchOut)]
     lib.ahs_last_error.restype = C.c_char_p
     lib.ahs_chain_cost.argtypes = [C.c_int64, C.c_int64, C.c_int64, C.c_int]
@@ -311,10 +328,18 @@ def phase_batch(batch: Batch, device: int = 0, devices=None, resident_iters: int
     valid until ahs_free_out); call .release() on the result before the next call on the same device.
     devices: list of CUDA ordinals -> ahs_phase_batch_multi (one contiguous, cost-balanced share of the chains per device).
     resident_iters > 0 -> ahs_phase_batch_resident (device-only timing over resident inputs).
+    batch.allele_dosage set -> ahs_phase_batch_genotyped on `device` or `devices` (not with resident_iters).
     """
     lib = load_library()
     s, o = batch.c_struct(), BatchOut()
-    if devices is not None:
+    if batch.allele_dosage is not None:
+        if resident_iters > 0:
+            raise ValueError("allele_dosage: the resident-input timing mode has no genotyped variant; "
+                             "phase without resident_iters, or set allele_dosage to None")
+        devs = list(devices) if devices is not None else [device]
+        arr = (C.c_int * len(devs))(*devs)
+        rc = lib.ahs_phase_batch_genotyped(C.byref(s), batch.dosage_ptr(), C.byref(o), arr, len(devs))
+    elif devices is not None:
         arr = (C.c_int * len(devices))(*devices)
         rc = lib.ahs_phase_batch_multi(C.byref(s), C.byref(o), arr, len(devices))
     elif resident_iters > 0:

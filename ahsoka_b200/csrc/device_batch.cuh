@@ -24,6 +24,7 @@ struct DB {
     const int64_t *bubble_off, *allele_off, *anode_off, *read_off, *entry_off, *enode_off;
     const int32_t *anode, *stage_a_order, *enode, *entry_read;
     const float   *entry_identity;
+    const uint8_t *allele_dosage;       // [NA] caller genotypes (ahs_phase_batch_genotyped), null without
     // ---- owner maps
     int32_t *bubble_chain, *allele_bubble, *entry_chain, *read_chain, *rankA;
     int64_t *mrow_off;                  // [C] chain offset into mask (u16 units)
@@ -54,6 +55,7 @@ struct DB {
     uint8_t *ch_small;                                    // [C] 1 = chain is scored + clustered out of shared memory (k_chain.cuh)
     // ---- consensus / threading
     PosRec *rec; uint16_t *back; int64_t *back_off; int32_t S_max;
+    uint64_t *gt_col;                                     // [NP] genotype key of each DP column (genotype_key, 0 = unknown), null without dosages
     int32_t *path; uint8_t *hap_allele; double *dp_cost;
     // ---- CSR cells out
     int64_t *cell_off; int32_t *cell_pos; uint8_t *cell_allele;

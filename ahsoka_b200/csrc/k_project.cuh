@@ -34,9 +34,19 @@ __global__ void k_owner(const int64_t* __restrict__ off, int n_owner, int64_t n_
 
 // ---------------------------------------------------------------- input validation (first kernel of every pass)
 // err_flags bits: 1 empty allele path, 2 more than 15 alleles, 4 offsets not monotone, 8 entry_read out of
-// range, 16 stage_a_order is not a permutation.  Every later kernel of phase 1 returns at once if a bit is set,
-// so a malformed batch can never drive an out-of-bounds access; the host reports the error after sync #1.
+// range, 16 stage_a_order is not a permutation, 32 the allele dosages of a bubble are neither all 0 nor sum to the
+// ploidy.  Every later kernel of phase 1 returns at once if a bit is set, so a malformed batch can never drive an
+// out-of-bounds access; the host reports the error after sync #1.
 #define AHS_BAIL_ON_ERR(d) do { if (*(volatile const int32_t*)(d).err_flags) return; } while (0)
+
+// Genotype of one bubble as one word: dosage of allele a in bits 4a..4a+3 (15 alleles x 4 bits; a valid dosage is at most
+// the ploidy, 6).  A DP state conforms iff the sum of 1 << 4 * allele over its haplotypes' consensus alleles equals the key:
+// the multiset test of rule R3.  `sum` = the bubble's dosage total; key 0 = genotype unknown.
+__device__ __forceinline__ uint64_t genotype_key(const uint8_t* __restrict__ dosage, int k, int& sum) {
+    uint64_t key = 0; sum = 0;
+    for (int a = 0; a < k; a++) { const uint32_t v = dosage[a]; sum += (int)v; key += (uint64_t)(v & 15u) << (4 * a); }
+    return key;
+}
 
 __global__ void k_validate(DB d, int32_t* __restrict__ max_k) {
     const int64_t stride = (int64_t)gridDim.x * blockDim.x, x0 = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -44,6 +54,10 @@ __global__ void k_validate(DB d, int32_t* __restrict__ max_k) {
     for (int64_t b = x0; b < d.NB; b += stride) {
         const int64_t k = d.allele_off[b + 1] - d.allele_off[b];
         if (k < 0) bad |= 4; else if (k > MAX_ALLELES) bad |= 2; else mk = max(mk, (int)k);
+        if (d.allele_dosage && k >= 0 && k <= MAX_ALLELES && d.allele_off[b] >= 0 && d.allele_off[b + 1] <= d.NA) {
+            int sum; genotype_key(d.allele_dosage + d.allele_off[b], (int)k, sum);
+            if (sum != 0 && sum != d.ploidy) bad |= 32;
+        }
     }
     for (int64_t a = x0; a < d.NA; a += stride) { const int64_t l = d.anode_off[a + 1] - d.anode_off[a]; if (l < 0) bad |= 4; else if (l == 0) bad |= 1; }
     for (int64_t e = x0; e < d.NE; e += stride) if (d.enode_off[e + 1] < d.enode_off[e]) bad |= 4;

@@ -173,6 +173,16 @@ constexpr int DP_THREADS = 128;
 
 __device__ __forceinline__ int ipow(int b, int e) { int r = 1; for (int i = 0; i < e; i++) r *= b; return r; }
 
+// caller genotypes (ahs_phase_batch_genotyped): the key of every DP column, from the dosages of its bubble (0 = unknown).
+// The dosages were validated by k_validate.
+__global__ void k_gt_columns(DB d) {
+    for (int64_t gp = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; gp < d.NP; gp += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t gb = d.bubble_off[d.pos_chain[gp]] + d.pos[gp];
+        int sum;
+        d.gt_col[gp] = genotype_key(d.allele_dosage + d.allele_off[gb], (int)(d.allele_off[gb + 1] - d.allele_off[gb]), sum);
+    }
+}
+
 __global__ void __launch_bounds__(DP_THREADS) k_thread(DB d, int32_t* __restrict__ work_counter) {
     extern __shared__ int32_t smem[];
     const int SM = d.S_max, p = d.ploidy;
@@ -181,6 +191,7 @@ __global__ void __launch_bounds__(DP_THREADS) k_thread(DB d, int32_t* __restrict
     int8_t* cc = (int8_t*)(Ab + SM);                    // covcost, -1 = not genotype conform
     __shared__ PosRec s_rec[2];
     __shared__ int s_chain;
+    __shared__ uint64_t s_gt;                           // genotype key of the column (caller genotypes only)
     const int tid = threadIdx.x, nt = blockDim.x;
     while (true) {
         if (tid == 0) s_chain = atomicAdd(work_counter, 1);
@@ -195,7 +206,7 @@ __global__ void __launch_bounds__(DP_THREADS) k_thread(DB d, int32_t* __restrict
         uint16_t* back = d.back + d.back_off[c];
         int kp = 0;
         for (int q = 0; q < n_pos; q++) {
-            if (tid == 0) s_rec[q & 1] = d.rec[p0 + q];
+            if (tid == 0) { s_rec[q & 1] = d.rec[p0 + q]; if (d.gt_col) s_gt = d.gt_col[p0 + q]; }
             __syncthreads();
             const PosRec& R = s_rec[q & 1];
             const PosRec& Rp = s_rec[(q & 1) ^ 1];
@@ -206,7 +217,9 @@ __global__ void __launch_bounds__(DP_THREADS) k_thread(DB d, int32_t* __restrict
             for (int t = tid; t < S; t += nt) {
                 int dig[MAX_PLOIDY]; { int x = t; for (int h = p - 1; h >= 0; h--) { dig[h] = x % kc; x /= kc; } }
                 bool conform;
-                if (p == 2) { const int a0 = R.cons_asc[dig[0]], a1 = R.cons_asc[dig[1]]; conform = (a0 == 0 && a1 == 1) || (a0 == 1 && a1 == 0); }
+                const uint64_t G = d.gt_col ? s_gt : 0; // 0: the built-in genotype rule
+                if (G) { uint64_t key = 0; for (int h = 0; h < p; h++) key += 1ull << (4 * R.cons_asc[dig[h]]); conform = key == G; }
+                else if (p == 2) { const int a0 = R.cons_asc[dig[0]], a1 = R.cons_asc[dig[1]]; conform = (a0 == 0 && a1 == 1) || (a0 == 1 && a1 == 0); }
                 else { conform = false; for (int h = 1; h < p; h++) conform |= R.cons_asc[dig[h]] != R.cons_asc[dig[0]]; }
                 int cost = 0;
                 for (int h = 0; h < p; h++) {
@@ -312,10 +325,13 @@ __global__ void __launch_bounds__(256) k_thread2(DB d, int32_t* __restrict__ wor
         if (n_pos == 0) continue;
         uint16_t* back = d.back + d.back_off[c];                       // 16 predecessor codes per position
         const uint32_t* recw = (const uint32_t*)(d.rec + p0);
-        uint32_t rw = lane < 22 ? recw[lane] : 0u;
+        // caller genotypes: lanes 22 and 23 carry the column's key (low, high word) next to the record
+        const uint32_t* gtw = d.gt_col ? (const uint32_t*)(d.gt_col + p0) : nullptr;
+        uint32_t rw = lane < 22 ? recw[lane] : (gtw && lane < 24) ? gtw[lane - 22] : 0u;
         int Dprev = DP_INF, gp0 = -1, gp1 = -1, kp = 0;
         for (int q = 0; q < n_pos; q++) {
-            const uint32_t rw_next = (q + 1 < n_pos && lane < 22) ? recw[(int64_t)(q + 1) * 22 + lane] : 0u;
+            uint32_t rw_next = (q + 1 < n_pos && lane < 22) ? recw[(int64_t)(q + 1) * 22 + lane] : 0u;
+            if (gtw && q + 1 < n_pos && (lane == 22 || lane == 23)) rw_next = gtw[(int64_t)(q + 1) * 2 + lane - 22];
             const uint32_t total = __shfl_sync(full, rw, 0);
             const int kc = (int)(__shfl_sync(full, rw, 1) & 0xffu);
             const int S = kc * kc;
@@ -325,7 +341,11 @@ __global__ void __launch_bounds__(256) k_thread2(DB d, int32_t* __restrict__ wor
             const uint32_t c0 = __shfl_sync(full, rw, 10 + d0), c1 = __shfl_sync(full, rw, 10 + d1);
             const int a0 = (int)((__shfl_sync(full, rw, 18 + (d0 >> 2)) >> (8 * (d0 & 3))) & 0xffu);
             const int a1 = (int)((__shfl_sync(full, rw, 18 + (d1 >> 2)) >> (8 * (d1 & 3))) & 0xffu);
-            const bool conform = (a0 == 0 && a1 == 1) || (a0 == 1 && a1 == 0);
+            bool conform;
+            if (gtw) {                                                 // key == (G ? G : 0x11): {0:1, 1:1} where the genotype is unknown
+                const uint64_t G = ((uint64_t)__shfl_sync(full, rw, 23) << 32) | __shfl_sync(full, rw, 22);
+                conform = (1ull << (4 * a0)) + (1ull << (4 * a1)) == (G ? G : 0x11ull);
+            } else conform = (a0 == 0 && a1 == 1) || (a0 == 1 && a1 == 0);
             const uint64_t m = d0 == d1 ? 2 : 1;
             int cost = 0;
             { const uint64_t lhs = (uint64_t)c0 * 4; if (lhs < (2 * m - 1) * total || lhs > (2 * m + 1) * total) cost++; }

@@ -61,7 +61,11 @@ __host__ __device__ inline size_t cn_smem_bytes() {
     return T * (4 + 2) * 2 + 1716 * 4 + 1716 + 2 * sizeof(PosRec) + 256;
 }
 
-__global__ void __launch_bounds__(CN_THREADS) k_thread_canon(DB d, CanonTables tb, int32_t* __restrict__ work_counter) {
+// GT: caller genotypes (d.gt_col) are present.  Two instances, so that the plain one is the kernel without any genotype code
+// (48 registers).  The GT instance declares 3 blocks per SM — what the 64 KB of shared memory of a block allows anyway —
+// because ptxas otherwise keeps it at 48 registers and spills; with the hint it takes 56 and spills nothing.
+template <bool GT>
+__global__ void __launch_bounds__(CN_THREADS, GT ? 3 : 0) k_thread_canon(DB d, CanonTables tb, int32_t* __restrict__ work_counter) {
     extern __shared__ __align__(16) unsigned char cn_sm[];
     const int p = d.ploidy;
     int32_t* Ev = (int32_t*)cn_sm; int32_t* Gv = Ev + 3003; int32_t* Dcur = Gv + 3003;
@@ -109,6 +113,22 @@ __global__ void __launch_bounds__(CN_THREADS) k_thread_canon(DB d, CanonTables t
                 }
                 cc[t] = conform ? (int8_t)cost : (int8_t)(-1 - cost);
                 any |= conform;
+            }
+            // caller genotype known at this column (ahs_phase_batch_genotyped): conformity is instead the multiset test of its
+            // key (genotype_key); every thread re-marks the states it has just written
+            if (GT) {
+                const uint64_t G = d.gt_col[p0 + q];
+                if (G) {
+                    any = 0;
+                    for (int t = tid; t < S; t += nt) {
+                        const uint32_t tp = tupc[tb.lvl[kc][p] + t];
+                        uint64_t key = 0;
+                        for (int h = 0; h < p; h++) key += 1ull << (4 * R.cons_asc[(tp >> (4 * h)) & 15u]);
+                        const int v = cc[t], cost = v >= 0 ? v : -1 - v;
+                        cc[t] = key == G ? (int8_t)cost : (int8_t)(-1 - cost);
+                        any |= key == G;
+                    }
+                }
             }
             any = __syncthreads_or(any);
             if (q == 0) {

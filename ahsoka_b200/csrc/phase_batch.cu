@@ -216,7 +216,8 @@ static Ctx* get_ctx(int device) {
     CK(cudaMemcpy(c->d_ln, ln.data(), 1025 * 8, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(c->d_ln1, ln1.data(), 1025 * 8, cudaMemcpyHostToDevice));
     CK(cudaFuncSetAttribute(k_thread, cudaFuncAttributeMaxDynamicSharedMemorySize, 21 * 4096 + 64));
-    CK(cudaFuncSetAttribute(k_thread_canon, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+    CK(cudaFuncSetAttribute(k_thread_canon<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+    CK(cudaFuncSetAttribute(k_thread_canon<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
     CK(cudaFuncSetAttribute(k_chain_front, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FR_SMEM_CAP));
     build_canon_tables(c->canon);
     c->smem_optin = prop.sharedMemPerBlockOptin;
@@ -280,6 +281,7 @@ static inline int grid_for(int64_t items, int per_block, int sms) {
 // ------------------------------------------------------------------ the pipeline
 struct Pipeline {
     Ctx* cx; Lane* ln; const ahs_batch_in* in; Sizes sz; DB d{};
+    const uint8_t* dosage = nullptr;                                            // caller genotypes of `in` (indexed like its allele_off), or null
     std::vector<int64_t> h_mrow_off, h_frow_off, h_pos_off, h_code_off, h_cw_off, h_back_off;
     int32_t *h_status = nullptr, *h_nfinal = nullptr, *h_npos = nullptr;      // pinned: D2H targets of sync #1
     int64_t* h_sc = nullptr;                                                   // pinned scalars of sync #1: cells, error flags, largest allele count
@@ -343,6 +345,7 @@ struct Pipeline {
         d.anode = up(in->anode, sz.NAN_); d.entry_read = up(in->entry_read, sz.NE);
         d.entry_identity = up(in->entry_identity, sz.NE);
         d.stage_a_order = in->stage_a_order ? up(in->stage_a_order, sz.NB) : nullptr;
+        d.allele_dosage = dosage ? up(dosage, sz.NA) : nullptr;
         h_mrow_off.assign(C, 0);
         int64_t acc = 0;
         for (int64_t c = 0; c < C; c++) {
@@ -513,6 +516,7 @@ struct Pipeline {
         if (h_err & 2) throw LimitFail{"a bubble has more than 15 alleles"};
         if (h_err & 8) throw ArgFail{"entry_read out of range"};
         if (h_err & 16) throw ArgFail{"stage_a_order is not a permutation"};
+        if (h_err & 32) throw ArgFail{"allele_dosage: the dosages of a bubble are neither all 0 nor sum to the ploidy"};
         sz.max_k = h_maxk;
         d.bits = sz.max_k <= 3 ? 2 : 4;
     }
@@ -622,6 +626,8 @@ struct Pipeline {
         if (NP) k_owner<<<grid_for(NP, TB, sms), TB, 0, st>>>(d.pos_off, (int)C, NP, d.pos_chain); n_launches += 1;
         if (NF) { if (sz.NB <= 96 * C) k_pack_rows<8><<<grid_for(NF, 32, sms), TB, 0, st>>>(d); else k_pack_rows<32><<<grid_for(NF, 8, sms), TB, 0, st>>>(d); n_launches += 1; }
         k_compact_pos<<<grid_for(C, 8, sms), TB, 0, st>>>(d); n_launches += 1;
+        d.gt_col = nullptr;
+        if (d.allele_dosage && NP) { d.gt_col = dalloc<uint64_t>(NP); k_gt_columns<<<grid_for(NP, TB, sms), TB, 0, st>>>(d); n_launches += 1; }
         // ---- CSR cells of the final matrix; with host output they travel D2H on a second stream under the clustering
         d.cell_base = cell_base;
         scan(d.fr_nv, NF, d.cell_off, cell_base);
@@ -729,7 +735,12 @@ struct Pipeline {
         CK(cudaEventRecord(ln->ev[5], st));
         if (NP && in->ploidy == 2) { k_thread2<<<(unsigned)std::min<int64_t>((C + 7) / 8, (int64_t)sms * 8), 256, 0, st>>>(d, counters + 1); n_launches += 1; }
         else if (NP && in->ploidy <= 4) { k_thread<<<std::min<int64_t>(C, (int64_t)sms * 8), DP_THREADS, 21 * (size_t)S_max + 64, st>>>(d, counters + 1); n_launches += 1; }
-        else if (NP) { k_thread_canon<<<std::min<int64_t>(C, (int64_t)sms * 4), CN_THREADS, 64 * 1024, st>>>(d, cx->canon, counters + 1); n_launches += 1; }
+        else if (NP) {
+            const unsigned grid = (unsigned)std::min<int64_t>(C, (int64_t)sms * 4);
+            if (d.gt_col) k_thread_canon<true><<<grid, CN_THREADS, 64 * 1024, st>>>(d, cx->canon, counters + 1);
+            else k_thread_canon<false><<<grid, CN_THREADS, 64 * 1024, st>>>(d, cx->canon, counters + 1);
+            n_launches += 1;
+        }
         CK(cudaEventRecord(ln->ev[6], st));
         CK(cudaGetLastError());
     }
@@ -811,7 +822,8 @@ struct ChainView {
     // the three rebased offset arrays live in page-locked staging: an async copy from pageable memory would first drain the
     // stream it is enqueued on (and with it the upload of the range before)
     ahs_batch_in v; int64_t *bubble_off = nullptr, *read_off = nullptr, *entry_off = nullptr;
-    void make(const ahs_batch_in* in, int64_t c0, int64_t c1, Pool& pin) {
+    const uint8_t* dosage = nullptr;                    // the caller's allele dosages from the range's first allele on, like anode_off
+    void make(const ahs_batch_in* in, const uint8_t* in_dosage, int64_t c0, int64_t c1, Pool& pin) {
         const int64_t C = in->n_chains, NB = in->bubble_off[C], NE = in->entry_off[C];
         const int64_t n = c1 - c0, b0 = in->bubble_off[c0], e0 = in->entry_off[c0];
         // the interior offsets dereferenced below are checked here; everything else is validated on the device
@@ -826,6 +838,7 @@ struct ChainView {
         v.n_chains = (int32_t)n; v.chain_id = in->chain_id ? in->chain_id + c0 : nullptr;
         v.bubble_off = bubble_off; v.read_off = read_off; v.entry_off = entry_off;
         v.allele_off = in->allele_off + b0; v.anode_off = in->anode_off + a0; v.anode = in->anode + an0;
+        dosage = in_dosage ? in_dosage + a0 : nullptr;
         v.stage_a_order = in->stage_a_order ? in->stage_a_order + b0 : nullptr;
         v.enode_off = in->enode_off + e0; v.enode = in->enode + en0;
         v.entry_read = in->entry_read + e0; v.entry_identity = in->entry_identity + e0;
@@ -851,7 +864,7 @@ static void alloc_out(ahs_batch_out* out, Ctx* cx, int64_t C, int p, int64_t NFt
 // uploads and projects under the clustering of range k, so that most of the H2D time is hidden), then — once the
 // caller has placed every range in the output arrays — the results are copied straight into their slices.
 struct DeviceJob {
-    Ctx* cx = nullptr; int device = -1; const ahs_batch_in* in = nullptr;
+    Ctx* cx = nullptr; int device = -1; const ahs_batch_in* in = nullptr; const uint8_t* dosage = nullptr;
     std::vector<Range> ranges;
     std::vector<ChainView> views; std::vector<Pipeline> pls; std::vector<Sizes> szs;
     std::unique_lock<std::mutex> lock;
@@ -860,8 +873,8 @@ struct DeviceJob {
     int iters = 0; int64_t* h_pairs = nullptr;
     HostTrace tr;
 
-    void begin(int dev, const ahs_batch_in* in_) {
-        device = dev; in = in_;
+    void begin(int dev, const ahs_batch_in* in_, const uint8_t* dosage_) {
+        device = dev; in = in_; dosage = dosage_;
         cx = get_ctx(device);
         lock = std::unique_lock<std::mutex>(cx->mu);
         tr.mark("context");
@@ -886,8 +899,8 @@ struct DeviceJob {
         auto prepare = [&](int k) {
             Pipeline& pl = pls[k];
             pl.cx = cx; pl.ln = &cx->lanes[k % N_LANES]; pl.early_out = iters == 0;
-            if (n == 1 && ranges[0].c0 == 0 && ranges[0].c1 == in->n_chains) { pl.in = in; pl.sz = validate(in); }
-            else { views[k].make(in, ranges[k].c0, ranges[k].c1, cx->pin); pl.in = &views[k].v; pl.sz = validate(pl.in, true); }
+            if (n == 1 && ranges[0].c0 == 0 && ranges[0].c1 == in->n_chains) { pl.in = in; pl.dosage = dosage; pl.sz = validate(in); }
+            else { views[k].make(in, dosage, ranges[k].c0, ranges[k].c1, cx->pin); pl.in = &views[k].v; pl.dosage = views[k].dosage; pl.sz = validate(pl.in, true); }
             szs[k] = pl.sz;
             if (pl.sz.C == 0) return;
             pl.upload(last_up);
@@ -1063,7 +1076,7 @@ struct ThreadBarrier {
 
 // one batch on the given devices.  G == 1: the whole batch on that device.  G > 1: plan_devices(); one host thread per
 // device; no inter-GPU traffic; every device writes its ranges straight into the (portable, page-locked) output arrays.
-static void phase_on_devices(const ahs_batch_in* in, ahs_batch_out* out, const int* devs, int G, int warmup, int iters) {
+static void phase_on_devices(const ahs_batch_in* in, const uint8_t* dosage, ahs_batch_out* out, const int* devs, int G, int warmup, int iters) {
     if (!out) throw ArgFail{"null output"};
     if (!devs || G < 1) throw ArgFail{"no devices"};
     for (int g = 0; g < G; g++) for (int h = 0; h < g; h++) if (devs[g] == devs[h]) throw ArgFail{"ahs_phase_batch_multi: a device id is listed twice"};
@@ -1076,7 +1089,7 @@ static void phase_on_devices(const ahs_batch_in* in, ahs_batch_out* out, const i
     const int64_t C = sz.C; const int p = in->ploidy;
     std::vector<DeviceJob> jobs(G);
     if (C == 0) {
-        jobs[0].begin(devs[0], in);
+        jobs[0].begin(devs[0], in, dosage);
         fill_empty_out(out, jobs[0].cx, p); jobs[0].cx->out_busy = true;
         jobs[0].lock.unlock();
         return;
@@ -1097,7 +1110,7 @@ static void phase_on_devices(const ahs_batch_in* in, ahs_batch_out* out, const i
     auto any_failed = [&]() { for (int g = 0; g < G; g++) if (rcs[g] != AHS_OK) return true; return false; };
     auto body = [&](int g) {
         DeviceJob& job = jobs[g];
-        rcs[g] = guarded("device", [&]() { job.begin(devs[g], in); job.ranges = plan[g]; job.enqueue(warmup, iters); });
+        rcs[g] = guarded("device", [&]() { job.begin(devs[g], in, dosage); job.ranges = plan[g]; job.enqueue(warmup, iters); });
         if (rcs[g] != AHS_OK) errs[g] = g_err;
         bar.arrive();
         if (g == 0 && !any_failed()) {
@@ -1206,15 +1219,19 @@ int ahs_plan_shares(const double* chain_cost, int64_t n_chains, int n_parts, int
 }
 
 int ahs_phase_batch(const ahs_batch_in* in, ahs_batch_out* out, int device) {
-    return guarded("ahs_phase_batch", [&]() { phase_on_devices(in, out, &device, 1, 0, 0); });
+    return guarded("ahs_phase_batch", [&]() { phase_on_devices(in, nullptr, out, &device, 1, 0, 0); });
 }
 
 int ahs_phase_batch_resident(const ahs_batch_in* in, ahs_batch_out* out, int device, int warmup, int iters) {
-    return guarded("ahs_phase_batch_resident", [&]() { phase_on_devices(in, out, &device, 1, warmup < 0 ? 0 : warmup, iters < 1 ? 1 : iters); });
+    return guarded("ahs_phase_batch_resident", [&]() { phase_on_devices(in, nullptr, out, &device, 1, warmup < 0 ? 0 : warmup, iters < 1 ? 1 : iters); });
 }
 
 int ahs_phase_batch_multi(const ahs_batch_in* in, ahs_batch_out* out, const int* device_ids, int n_devices) {
-    return guarded("ahs_phase_batch_multi", [&]() { phase_on_devices(in, out, device_ids, n_devices, 0, 0); });
+    return guarded("ahs_phase_batch_multi", [&]() { phase_on_devices(in, nullptr, out, device_ids, n_devices, 0, 0); });
+}
+
+int ahs_phase_batch_genotyped(const ahs_batch_in* in, const uint8_t* allele_dosage, ahs_batch_out* out, const int* device_ids, int n_devices) {
+    return guarded("ahs_phase_batch_genotyped", [&]() { phase_on_devices(in, allele_dosage, out, device_ids, n_devices, 0, 0); });
 }
 
 int ahs_debug_std_sort(int32_t* keys, int32_t* values, int32_t n, int descending, int device) {

@@ -97,3 +97,13 @@ def generate(p: SynthParams, gfa_gaf_prefix: str | None = None) -> Batch:
         return b
     finally:
         lib.ahs_synth_free(h)
+
+
+def true_dosage(batch: Batch) -> np.ndarray:
+    """Per-allele dosages of the generator's haplotypes (batch.truth["hap_allele"]), indexed like allele_off: the number of
+    haplotypes that carry each allele of each bubble.  Every haplotype gets a distinct allele while the bubble has at least
+    ploidy alleles (diploid truth is always {0:1, 1:1}); the remaining haplotypes draw one at random."""
+    p = int(batch.ploidy)
+    hap = batch.truth["hap_allele"].reshape(-1, p).astype(np.int64)
+    idx = batch.allele_off[:-1, None] + hap
+    return np.bincount(idx.ravel(), minlength=int(batch.allele_off[-1])).astype(np.uint8)

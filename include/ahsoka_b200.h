@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define AHS_ABI_VERSION 2
+#define AHS_ABI_VERSION 3   /* 3: ahs_phase_batch_genotyped */
 
 /* Return codes of the entry points. */
 #define AHS_OK              0
@@ -156,6 +156,27 @@ int  ahs_phase_batch(const ahs_batch_in *in, ahs_batch_out *out, int device);
  */
 int  ahs_phase_batch_multi(const ahs_batch_in *in, ahs_batch_out *out,
                            const int *device_ids, int n_devices);
+
+/*
+ * Phase one batch with caller-supplied genotypes.  n_devices == 1: as ahs_phase_batch on
+ * device_ids[0]; more: as ahs_phase_batch_multi, with the same shares.
+ *
+ * allele_dosage[n_alleles] is indexed like allele_off: allele a of global bubble gb is entry
+ * allele_off[gb] + a, and holds the number of haplotypes that carry that allele.  Per bubble, either
+ * every dosage is 0 (genotype unknown) or the dosages sum to `ploidy`; anything else, at any bubble
+ * (trivial chains and bubbles no read covers included), fails the whole call with AHS_ERR_ARG and a
+ * message naming allele_dosage, and no chain is phased.
+ *
+ * Where the genotype of a covered position is known, the threading DP allows only the states whose
+ * multiset of consensus alleles equals {a: dosage[a] : dosage[a] > 0} (the consensus the threader
+ * receives: clusters in ascending id order); where it is unknown the built-in rule applies
+ * ({0:1, 1:1} at ploidy 2, "the consensus alleles are not all equal" above).  If no state of a
+ * column conforms, every state is allowed.  Costs and tie rules are those of ahs_phase_batch, so the
+ * emitted hap_allele multiset may still differ from the genotype.  allele_dosage == NULL, or all
+ * zero, gives the result of ahs_phase_batch / ahs_phase_batch_multi bit for bit.
+ */
+int  ahs_phase_batch_genotyped(const ahs_batch_in *in, const uint8_t *allele_dosage,
+                               ahs_batch_out *out, const int *device_ids, int n_devices);
 
 /*
  * Resident-input variant used for device-only timing: upload once, run the kernels
